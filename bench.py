@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — env-steps/s of batched CubicEnv.step on B200 (BASELINE.json metric), one JSON line on stdout.
 
-    python bench.py [--gpus N --steps K --warmup W] [--workload c4|c2|c3] [--impl reference]
+    python bench.py [--gpus N --steps K --warmup W] [--workload c4|c2|c3] [--impl reference] [--dump-outputs DIR]
 
 A "step" is ONE nav3d_step launch over every env of the workload (one pass of the hot path over one batch):
   value     device-resident: actions already in HBM, observations written into an HBM rollout ring; CUDA-event timed
@@ -246,6 +246,29 @@ def timed_steps(eng, buf, steps, torch, dist, world):
     return ms, ms_local, eng.launch_count - l0
 
 
+DUMP_MAX_ENVS = 1 << 17            # 2^17 envs x (80 + 3) f32 + f64 id = 44.6 MB, under the 64 MB a dump may take
+
+
+def dump_outputs(out_dir, buf, torch):
+    """Writes what the last timed nav3d_step returned to its caller (observation, reward, terminated, truncated) as
+    float32 .npy files, for the envs of a fixed sample (seeded, the same in every run: all envs when at most
+    DUMP_MAX_ENVS), plus their env ids (float64).  Two builds run with the same arguments can be compared file for
+    file."""
+    import numpy as np
+    n = buf.rew.shape[0]
+    if n <= DUMP_MAX_ENVS:
+        idx = np.arange(n)
+    else:
+        idx = np.sort(np.random.default_rng(0).choice(n, DUMP_MAX_ENVS, replace=False))
+    tid = torch.as_tensor(idx, device=buf.rew.device)
+    arrays = {"obs": buf.last_obs()[tid], "reward": buf.rew[tid], "terminated": buf.te[tid], "truncated": buf.tr[tid]}
+    out_dir = Path(out_dir)
+    out_dir.mkdir(parents=True, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(out_dir / f"{name}.npy", t.cpu().numpy().astype(np.float32))
+    np.save(out_dir / "env_ids.npy", idx.astype(np.float64))
+
+
 def time_steps(eng, n, steps, warmup, torch, dist, world, lanes_note=None, ring=4, act_rows=16, seed=0):
     """Reset, `warmup` untimed steps, `steps` timed ones.  Returns (ms_total_max_over_ranks, ms_total_local, launches)."""
     buf = StepBuffers(eng, n, torch, ring, act_rows, seed)
@@ -467,7 +490,14 @@ def main():
     ap.add_argument("--e2e-steps", type=int, default=10)
     ap.add_argument("--preroll", type=int, default=600,
                     help="untimed fused random steps before the second, mid-episode measurement (0 = skip it)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what their last step returned (obs, reward, terminated, truncated "
+                         "of a fixed sample of rank 0's envs, and the sample's env ids) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs saves what the GPU path's timed steps returned; the reference arm has none to save")
     args.warmup = max(args.warmup, 3)
     if args.impl == "reference":
         run_reference(args)
@@ -513,6 +543,8 @@ def main():
         buf.step(eng)
     ms, ms_local, launches = timed_steps(eng, buf, args.steps, torch, dist, world)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, buf, torch)
     value = n_total * args.steps / (ms / 1e3)
     regime = "cold" if args.warmup + args.steps < 200 else "steady"
     check = None

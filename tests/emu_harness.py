@@ -8,6 +8,8 @@ import numpy as np
 
 import os
 
+from __graft_entry__ import find_nvcc
+
 HERE = Path(__file__).resolve().parent / "emu"
 ASAN = os.environ.get("NAV3D_EMU_ASAN") == "1"          # tools/emu_asan.sh: the same source under AddressSanitizer + UBSan
 LIB = HERE / ("libnav3d_emu_asan.so" if ASAN else "libnav3d_emu.so")
@@ -21,7 +23,7 @@ def build():
         if not LIB.exists() or LIB.stat().st_mtime < max(src.stat().st_mtime, CORE.stat().st_mtime):
             extra = (["-g", "-DNAV3D_EMU_ASAN", "-Xcompiler", "-fsanitize=address", "-Xcompiler", "-fsanitize=undefined", "-Xcompiler",
                       "-fno-omit-frame-pointer", "-Xcompiler", "-fno-sanitize-recover=undefined"] if ASAN else [])
-            subprocess.check_call(["nvcc", "-O2", "-std=c++17", "-Wno-deprecated-gpu-targets", "-shared", "-Xcompiler",
+            subprocess.check_call([find_nvcc(), "-O2", "-std=c++17", "-Wno-deprecated-gpu-targets", "-shared", "-Xcompiler",
                                    "-fPIC", *extra, "-o", str(LIB), str(src)], stdout=subprocess.DEVNULL)
 
 

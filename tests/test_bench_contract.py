@@ -1,9 +1,13 @@
 """bench.py's output contract: the committed GPU line (profiles/bench_r02.json, produced on a B200) and a live run of the
 reference arm on this machine's cores carry every key the driver reads, with consistent values."""
+import importlib.util
 import json
 import subprocess
 import sys
 import textwrap
+
+import numpy as np
+import pytest
 
 from conftest import ROOT
 
@@ -88,3 +92,88 @@ def test_reference_arm_does_not_map_the_product_library():
     out = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=600, cwd=str(ROOT))
     assert out.returncode == 0, out.stderr[-2000:]
     assert "MAPPED []" in out.stdout
+
+
+def load_bench():
+    spec = importlib.util.spec_from_file_location("bench_under_test", ROOT / "bench.py")
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    return bench
+
+
+def test_dump_outputs_sample_fits_and_matches_env_ids(tmp_path):
+    """--dump-outputs at the flagship size (2^20 envs): a fixed sample, under 64 MB, every row the one of its env id."""
+    import torch
+    bench = load_bench()
+
+    class Buf:
+        pass
+    n = 1 << 20
+    buf = Buf()
+    buf.rew = torch.arange(n, dtype=torch.float32) * 0.5
+    buf.te = (torch.arange(n) % 3 == 0).to(torch.uint8)
+    buf.tr = (torch.arange(n) % 5 == 0).to(torch.uint8)
+    obs = torch.arange(n, dtype=torch.float32)[:, None].expand(n, 80)       # row i holds i, without 335 MB
+    buf.last_obs = lambda: obs
+    for d in ("a", "b"):
+        bench.dump_outputs(tmp_path / d, buf, torch)
+    files = sorted(p.name for p in (tmp_path / "a").iterdir())
+    assert files == ["env_ids.npy", "obs.npy", "reward.npy", "terminated.npy", "truncated.npy"]
+    assert sum(p.stat().st_size for p in (tmp_path / "a").iterdir()) <= 64 << 20
+    got = {f[:-4]: np.load(tmp_path / "a" / f) for f in files}
+    for f in files:
+        assert got[f[:-4]].dtype in (np.float32, np.float64)
+        assert np.array_equal(got[f[:-4]], np.load(tmp_path / "b" / f))                    # the same sample every run
+    ids = got["env_ids"].astype(np.int64)
+    assert len(ids) == bench.DUMP_MAX_ENVS and len(np.unique(ids)) == len(ids) and ids.max() < n
+    assert np.array_equal(got["obs"], np.repeat(ids[:, None].astype(np.float32), 80, axis=1))
+    assert np.array_equal(got["reward"], ids * 0.5)
+    assert np.array_equal(got["terminated"], (ids % 3 == 0).astype(np.float32))
+    assert np.array_equal(got["truncated"], (ids % 5 == 0).astype(np.float32))
+
+
+def test_dump_outputs_is_refused_for_the_reference_arm(tmp_path):
+    out = subprocess.run([sys.executable, str(ROOT / "bench.py"), "--impl", "reference", "--dump-outputs", str(tmp_path)],
+                         capture_output=True, text=True, timeout=600, cwd=str(ROOT))
+    assert out.returncode == 2 and "--dump-outputs" in out.stderr and not any(tmp_path.iterdir())
+
+
+@pytest.mark.gpu
+def test_dump_outputs_hold_what_the_last_timed_step_returned(tmp_path):
+    """Two runs with the same arguments time exactly --steps launches and dump the same arrays, and those are what the
+    last timed step returned: the C oracle, replaying bench.py's actions from the same reset, gives every row bit for
+    bit (an off-by-one ring slot, or an array read before the last launch finished, would not)."""
+    import types
+
+    import torch
+    from oracle import c_oracle
+    W, K, n = 3, 7, 4096                                                     # workload c2: 4096 envs, all dumped
+    outs = []
+    for d in ("a", "b"):
+        out = subprocess.run([sys.executable, str(ROOT / "bench.py"), "--workload", "c2", "--steps", str(K), "--warmup", str(W),
+                              "--no-extras", "--preroll", "0", "--e2e-steps", "3", "--dump-outputs", str(tmp_path / d)],
+                             capture_output=True, text=True, timeout=600, cwd=str(ROOT))
+        assert out.returncode == 0, out.stderr[-2000:]
+        line = json.loads(out.stdout.strip().splitlines()[-1])
+        assert line["steps"] == K and line["gpu_launches"] == K and line["check"]["steps_replayed"] == W + K
+        outs.append({p.stem: np.load(p) for p in (tmp_path / d).iterdir()})
+    a, b = outs
+    assert set(a) == {"env_ids", "obs", "reward", "terminated", "truncated"}
+    assert np.array_equal(a["env_ids"], np.arange(n)) and a["obs"].shape == (n, 80)
+    for k in a:
+        assert a[k].dtype in (np.float32, np.float64) and np.array_equal(a[k], b[k], equal_nan=True)
+
+    bench = load_bench()
+    # the action rows bench.py drew: its StepBuffers on the same device, min(1024, W + 2K) rows as main() asks for
+    stand_in = types.SimpleNamespace(device=torch.device("cuda", 0), obs_dim=80)
+    actions = bench.StepBuffers(stand_in, n, torch, act_rows=min(1024, W + 2 * K)).actions.cpu().numpy()
+    spec = bench.workload_spec("c2")
+    rooms = bench.load_rooms(spec)
+    ov = c_oracle.OracleVec(n, [c_oracle.OracleRoom(r.grid, -2) for r in rooms], spec["L"], -2.0, 2024, 0, True)  # main()'s seed
+    ov.reset()
+    for t in range(W + K):
+        ov.step(actions[t % len(actions)])
+    assert np.array_equal(a["obs"].view(np.uint32), ov.obs.view(np.uint32))
+    assert np.array_equal(a["reward"], ov.reward.astype(np.float32))
+    assert np.array_equal(a["terminated"], ov.terminated.astype(np.float32))
+    assert np.array_equal(a["truncated"], ov.truncated.astype(np.float32))

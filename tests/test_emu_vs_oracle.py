@@ -1,15 +1,14 @@
 """Host-side check of the packed-representation logic (csrc/nav3d_core.cuh compiled for the CPU, one lane per env)
 against the oracle.  This is a debugging aid for the GPU-less container; the parity tests proper are -m gpu."""
-import shutil
-
 import numpy as np
 import pytest
 
+from __graft_entry__ import find_nvcc
 from conftest import ROOMS
 from lockstep import compare_grids, compare_step
 from nav3d.rooms import load_room_dir, load_room_file
 
-pytestmark = pytest.mark.skipif(shutil.which("nvcc") is None, reason="nvcc needed to build the host emulation")
+pytestmark = pytest.mark.skipif(find_nvcc() is None, reason="nvcc needed to build the host emulation")
 
 
 def run_lockstep(oracle, rooms, n, L, steps, seed, auto_reset=True, crash=-2.0, check_state_every=1, lanes=1,
