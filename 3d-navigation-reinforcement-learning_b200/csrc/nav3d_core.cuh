@@ -1159,4 +1159,166 @@ NAV3D_HD bool simple_step_env(const EngineParams &P, const StepIO &io, int env, 
     return will_reset;
 }
 
+// ---------------------------------------------------------------------------------------------------------------
+// env-state blobs (nav3d_save_envs / nav3d_load_envs): the complete state of one env, self-describing, fixed size.
+//   [0, 32)          BlobHeader
+//   [32, 64)         EnvState, unchanged
+//   [64, know_off)   the env's current observation row (obs_dim f32), padded to a multiple of 16 bytes (padding not written)
+//   [know_off, +env_stride)  the knowledge block with the engine's own offsets: K at 0, overflow bytes at ovf_off.  Only the
+//                    live part of the blob's room is written: k_bytes (simpleEnv k2_bytes) of K and W*D*H overflow bytes —
+//                    the range a reset clears and a step can read.
+// The per-env copy is split over `nl` lanes (lane = 0 .. nl-1); the device kernels run it with a warp per env, the host
+// emulation with one lane.
+// ---------------------------------------------------------------------------------------------------------------
+constexpr uint32_t kBlobMagic = 0x4e334445u;     // "ED3N" little-endian
+constexpr uint32_t kBlobVersion = 1u;
+constexpr uint32_t kBlobObsOff = 64;
+constexpr uint8_t kBlobLoaded = 0, kBlobBadEnv = 1, kBlobInvalid = 2;   // nav3d_load_envs status codes
+
+struct alignas(16) BlobHeader {
+    uint32_t magic, version;
+    unsigned long long signature;  // engine signature (nav3d_load_rooms): env kind, L, env_stride and the room table
+    uint32_t room;                 // == EnvState::room
+    uint32_t k_live, ovf_live;     // bytes of K and of the overflow volume the blob holds
+    uint32_t obs_dim;
+};
+static_assert(sizeof(BlobHeader) == 32, "blob header");
+
+NAV3D_HD bool simple_kind(const EngineParams &P) { return P.obs_dim != kObsDim; }
+NAV3D_HD unsigned long long blob_know_off(const EngineParams &P) {
+    return kBlobObsOff + (((unsigned long long)P.obs_dim * 4u + 15u) & ~15ull);
+}
+NAV3D_HD unsigned long long blob_bytes(const EngineParams &P) { return blob_know_off(P) + P.env_stride; }
+NAV3D_HD uint32_t blob_k_live(const EngineParams &P, const RoomDev &R) { return simple_kind(P) ? k2_bytes(R) : k_bytes(R); }
+NAV3D_HD uint32_t blob_ovf_live(const EngineParams &P, const RoomDev &R) {
+    return simple_kind(P) ? 0u : (uint32_t)R.W * R.D * R.H;
+}
+
+NAV3D_HD uint4 load_stream(const uint4 *p) {
+#ifdef __CUDA_ARCH__
+    return __ldcs(p);
+#else
+    return *p;
+#endif
+}
+NAV3D_HD void store_stream(uint4 *p, uint4 v) {
+#ifdef __CUDA_ARCH__
+    __stcs(p, v);
+#else
+    *p = v;
+#endif
+}
+
+// n bytes from src to dst, both 16-byte aligned: 16-byte copies (four in flight per lane), then the < 16 tail bytes.
+// STREAM_LD / STREAM_ST: evict-first hint on the blob side.
+template <bool STREAM_LD, bool STREAM_ST>
+NAV3D_HD void copy_live(uint8_t *dst, const uint8_t *src, uint32_t n, int lane, int nl) {
+    const uint4 *s4 = reinterpret_cast<const uint4 *>(src);
+    uint4 *d4 = reinterpret_cast<uint4 *>(dst);
+    const uint32_t n16 = n >> 4;
+    uint32_t i = (uint32_t)lane;
+    for (; i + 3u * nl < n16; i += 4u * nl) {
+        uint4 v[4];
+#pragma unroll
+        for (int j = 0; j < 4; j++) v[j] = STREAM_LD ? load_stream(s4 + i + j * nl) : s4[i + j * nl];
+#pragma unroll
+        for (int j = 0; j < 4; j++) {
+            if (STREAM_ST) store_stream(d4 + i + j * nl, v[j]);
+            else d4[i + j * nl] = v[j];
+        }
+    }
+    for (; i < n16; i += nl) {
+        const uint4 v = STREAM_LD ? load_stream(s4 + i) : s4[i];
+        if (STREAM_ST) store_stream(d4 + i, v);
+        else d4[i] = v;
+    }
+    for (uint32_t b = (n16 << 4) + (uint32_t)lane; b < n; b += nl) dst[b] = src[b];
+}
+
+// One observation row (obs_dim f32; 16-byte aligned rows of CubicEnv move as float4, simpleEnv rows as f32)
+template <bool STREAM_ST>
+NAV3D_HD void copy_row(float *dst, const float *src, int obs_dim, int lane, int nl) {
+    if ((obs_dim & 3) == 0 && ((reinterpret_cast<uintptr_t>(dst) | reinterpret_cast<uintptr_t>(src)) & 15u) == 0) {
+        for (int i = lane; i < obs_dim / 4; i += nl) {
+            const float4 v = reinterpret_cast<const float4 *>(src)[i];
+            if (STREAM_ST) store_stream(reinterpret_cast<float4 *>(dst) + i, v);
+            else reinterpret_cast<float4 *>(dst)[i] = v;
+        }
+    } else {
+        for (int i = lane; i < obs_dim; i += nl) {
+            if (STREAM_ST) store_stream(dst + i, src[i]);
+            else dst[i] = src[i];
+        }
+    }
+}
+
+// save: env -> blob.  An env id outside 0..n_envs-1 gets a header with magic 0, which every load rejects.
+NAV3D_HD void save_env_lane(const EngineParams &P, unsigned long long sig, int env, const float *obs, uint8_t *blob, int lane,
+                            int nl) {
+    BlobHeader *h = reinterpret_cast<BlobHeader *>(blob);
+    if (env < 0 || env >= P.n_envs) {
+        if (lane == 0) { BlobHeader z{}; *h = z; }
+        return;
+    }
+    const EnvState st = P.states[env];
+    const RoomDev R = P.rooms[st.room];
+    const uint32_t k_live = blob_k_live(P, R), ovf_live = blob_ovf_live(P, R);
+    if (lane == 0) {
+        BlobHeader hd;
+        hd.magic = kBlobMagic; hd.version = kBlobVersion; hd.signature = sig; hd.room = st.room;
+        hd.k_live = k_live; hd.ovf_live = ovf_live; hd.obs_dim = (uint32_t)P.obs_dim;
+        *h = hd;
+        *reinterpret_cast<EnvState *>(blob + sizeof(BlobHeader)) = st;
+    }
+    copy_row<true>(reinterpret_cast<float *>(blob + kBlobObsOff), obs + (unsigned long long)env * P.obs_dim, P.obs_dim, lane, nl);
+    const uint8_t *envk = P.know + (unsigned long long)env * P.env_stride;
+    uint8_t *bk = blob + blob_know_off(P);
+    copy_live<false, true>(bk, envk, k_live, lane, nl);
+    if (ovf_live) copy_live<false, true>(bk + P.ovf_off, envk + P.ovf_off, ovf_live, lane, nl);
+}
+
+// load, part 1: may `blob` be loaded into `env` of this engine?  Reads the header and the record only.
+NAV3D_HD uint8_t blob_status(const EngineParams &P, unsigned long long sig, int env, const uint8_t *blob) {
+    if (env < 0 || env >= P.n_envs) return kBlobBadEnv;
+    const BlobHeader h = *reinterpret_cast<const BlobHeader *>(blob);
+    if (h.magic != kBlobMagic || h.version != kBlobVersion || h.signature != sig || h.room >= (uint32_t)P.n_rooms ||
+        h.obs_dim != (uint32_t)P.obs_dim)
+        return kBlobInvalid;
+    const RoomDev R = P.rooms[h.room];
+    const EnvState st = *reinterpret_cast<const EnvState *>(blob + sizeof(BlobHeader));
+    if (h.k_live != blob_k_live(P, R) || h.ovf_live != blob_ovf_live(P, R) || st.room != h.room || st.x >= R.W ||
+        st.y >= R.D || st.z >= R.H)
+        return kBlobInvalid;
+    return kBlobLoaded;
+}
+
+// load, part 2 (a blob that blob_status accepted): blob -> env, and the blob's observation row -> obs.
+NAV3D_HD void load_env_lane(const EngineParams &P, int env, const uint8_t *blob, float *obs, int lane, int nl) {
+    const BlobHeader h = *reinterpret_cast<const BlobHeader *>(blob);
+    uint8_t *envk = P.know + (unsigned long long)env * P.env_stride;
+    const uint8_t *bk = blob + blob_know_off(P);
+    copy_live<true, false>(envk, bk, h.k_live, lane, nl);
+    if (h.ovf_live) copy_live<true, false>(envk + P.ovf_off, bk + P.ovf_off, h.ovf_live, lane, nl);
+    copy_row<true>(obs + (unsigned long long)env * P.obs_dim, reinterpret_cast<const float *>(blob + kBlobObsOff), P.obs_dim,
+                   lane, nl);
+    if (lane == 0) P.states[env] = *reinterpret_cast<const EnvState *>(blob + sizeof(BlobHeader));
+}
+
+// Engine signature (host side, nav3d_load_rooms): FNV-1a 64 over the env kind, L, env_stride and, per room, its dims, wall
+// code, dense grid and the start cell it resets to (0xffffffff: random).  Lanes, seed, env_id0 and the reward parameters
+// are deliberately not part of it: blobs move between engines that differ only in those.
+inline unsigned long long sig_bytes(unsigned long long h, const void *p, size_t n) {
+    const uint8_t *b = static_cast<const uint8_t *>(p);
+    for (size_t i = 0; i < n; i++) { h ^= b[i]; h *= 0x100000001b3ull; }
+    return h;
+}
+inline unsigned long long sig_engine(int kind, int L, unsigned long long env_stride) {
+    const int32_t v[2] = {kind, L};
+    return sig_bytes(sig_bytes(0xcbf29ce484222325ull, v, sizeof v), &env_stride, sizeof env_stride);
+}
+inline unsigned long long sig_room(unsigned long long h, int W, int D, int H, int wall_code, const int8_t *grid, uint32_t start) {
+    const int32_t v[5] = {W, D, H, wall_code, (int32_t)start};
+    return sig_bytes(sig_bytes(h, v, sizeof v), grid, (size_t)W * D * H);
+}
+
 }  // namespace nav3d

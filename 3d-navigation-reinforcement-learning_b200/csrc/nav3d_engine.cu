@@ -629,6 +629,32 @@ __global__ void init_states_kernel(EnvState *states, int n) {
     states[i] = s;
 }
 
+// Env-state blobs, a warp per listed env (nav3d_core.cuh save_env_lane / load_env_lane).  A pure copy of the live part of
+// the env's block: HBM-bound.  Blob stores (save) and blob loads (load) carry the evict-first hint, so that a large save or
+// load does not push the knowledge lines of a running rollout out of L2.
+__global__ void __launch_bounds__(kBlock) save_envs_kernel(const __grid_constant__ EngineParams P, unsigned long long sig,
+                                                           const int32_t *__restrict__ env_ids, int n,
+                                                           const float *__restrict__ obs, uint8_t *blobs,
+                                                           unsigned long long blob_bytes) {
+    const long long i = ((long long)blockIdx.x * kBlock + threadIdx.x) >> 5;
+    if (i >= n) return;
+    const int env = env_ids ? env_ids[i] : (int)i;
+    save_env_lane(P, sig, env, obs, blobs + (unsigned long long)i * blob_bytes, threadIdx.x & 31, 32);
+}
+__global__ void __launch_bounds__(kBlock) load_envs_kernel(const __grid_constant__ EngineParams P, unsigned long long sig,
+                                                           const int32_t *__restrict__ env_ids, int n,
+                                                           const uint8_t *blobs, unsigned long long blob_bytes, float *obs,
+                                                           uint8_t *status) {
+    const long long i = ((long long)blockIdx.x * kBlock + threadIdx.x) >> 5;
+    if (i >= n) return;
+    const int lane = threadIdx.x & 31;
+    const int env = env_ids ? env_ids[i] : (int)i;
+    const uint8_t *blob = blobs + (unsigned long long)i * blob_bytes;
+    const uint8_t st = blob_status(P, sig, env, blob);      // the whole header is checked before anything is written
+    if (status && lane == 0) status[i] = st;
+    if (st == kBlobLoaded) load_env_lane(P, env, blob, obs, lane, 32);
+}
+
 size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
 }  // namespace
@@ -659,7 +685,8 @@ struct nav3d_engine {
     int simple_stride = 0;      // simpleEnv, lanes_per_env == 1: floats per staged row (odd: conflict-free), 0 = not staged
     bool tpe_staged = true;     // thread-per-env kernels: rows staged in shared memory, marking by the warp (NAV3D_TPE_STAGED)
     int tpe_block = 64;         // their CTA size (NAV3D_TPE_BLOCK)
-    bool reset_seen = false;    // a nav3d_reset call has been made since the rooms were loaded
+    bool reset_seen = false;    // a nav3d_reset (or nav3d_restore / nav3d_load_envs) call has been made since the rooms were loaded
+    unsigned long long signature = 0;   // engine signature of env-state blobs (nav3d_core.cuh sig_engine / sig_room)
     bool pdl = true;            // programmatic dependent launch of the step kernel (NAV3D_PDL=0 switches it off)
     float *d_dist_lut = nullptr;
     cudaStream_t own_stream = nullptr;
@@ -933,6 +960,10 @@ int nav3d_load_rooms(nav3d_engine *e, int32_t n_rooms, const nav3d_room_desc *ro
         }
     e->h_rooms = hr;
     e->know_bytes = know_bytes;
+    e->signature = sig_engine(e->cfg.env_kind, e->cfg.local_map_length, stride);
+    for (int i = 0; i < n_rooms; i++)
+        e->signature = sig_room(e->signature, rooms[i].width, rooms[i].depth, rooms[i].height, rooms[i].wall_code,
+                                rooms[i].grid, start[(size_t)i]);
     e->room_bytes = sizeof(RoomDev) * n_rooms + 2 * n_occz + 8 * n_occ64 + 4 * n_free_cap;
     EngineParams &P = e->P;
     P.rooms = e->d_rooms; P.occz = e->d_occz; P.occ64 = e->d_occ64; P.free_cells = e->d_free;
@@ -1220,6 +1251,48 @@ int nav3d_restore(nav3d_engine *e, const void *host_buf, size_t bytes) {
     CUDA_TRY(cudaMemcpy(e->d_states, host_buf, sb, cudaMemcpyHostToDevice));
     CUDA_TRY(cudaMemcpy(e->d_know, (const char *)host_buf + sb, e->know_bytes, cudaMemcpyHostToDevice));
     e->reset_seen = true;
+    return NAV3D_OK;
+}
+
+size_t nav3d_env_state_bytes(const nav3d_engine *e) {
+    if (!e || e->h_rooms.empty()) return 0;
+    return (size_t)blob_bytes(e->P);
+}
+
+int nav3d_save_envs(nav3d_engine *e, const int32_t *env_ids, int32_t n, const float *obs, void *blobs, void *stream) {
+    if (n < 0) return fail(NAV3D_ERR_INVALID, "n must be >= 0");
+    if (!obs || !blobs) return fail(NAV3D_ERR_INVALID, "obs and blobs are required");
+    if (((uintptr_t)blobs & 15u)) return fail(NAV3D_ERR_INVALID, "blobs must be 16-byte aligned");
+    if (int rc = check_steppable(e)) return rc;
+    if (!env_ids && n > e->cfg.n_envs) return fail(NAV3D_ERR_INVALID, "n out of range");
+    if (!e->simple && ((uintptr_t)obs & 15u)) return fail(NAV3D_ERR_INVALID, "obs must be 16-byte aligned");
+    if (n == 0) return NAV3D_OK;
+    NAV3D_DEVICE(e);
+    NvtxRange range("nav3d_save_envs");
+    save_envs_kernel<<<grid_for(n, 32), kBlock, 0, (cudaStream_t)stream>>>(e->P, e->signature, env_ids, n, obs,
+                                                                              static_cast<uint8_t *>(blobs), blob_bytes(e->P));
+    e->launches++;
+    CUDA_TRY(cudaGetLastError());
+    return NAV3D_OK;
+}
+
+int nav3d_load_envs(nav3d_engine *e, const int32_t *env_ids, int32_t n, const void *blobs, float *obs, uint8_t *status,
+                    void *stream) {
+    if (n < 0) return fail(NAV3D_ERR_INVALID, "n must be >= 0");
+    if (!obs || !blobs) return fail(NAV3D_ERR_INVALID, "obs and blobs are required");
+    if (((uintptr_t)blobs & 15u)) return fail(NAV3D_ERR_INVALID, "blobs must be 16-byte aligned");
+    if (int rc = check_ready(e)) return rc;
+    if (!env_ids && n > e->cfg.n_envs) return fail(NAV3D_ERR_INVALID, "n out of range");
+    if (!e->simple && ((uintptr_t)obs & 15u)) return fail(NAV3D_ERR_INVALID, "obs must be 16-byte aligned");
+    if (n == 0) return NAV3D_OK;
+    NAV3D_DEVICE(e);
+    NvtxRange range("nav3d_load_envs");
+    e->reset_seen = true;
+    load_envs_kernel<<<grid_for(n, 32), kBlock, 0, (cudaStream_t)stream>>>(e->P, e->signature, env_ids, n,
+                                                                              static_cast<const uint8_t *>(blobs),
+                                                                              blob_bytes(e->P), obs, status);
+    e->launches++;
+    CUDA_TRY(cudaGetLastError());
     return NAV3D_OK;
 }
 

@@ -17,6 +17,7 @@ OBS_DIM = 80
 STATE_INTS = 16
 ENV_CUBIC, ENV_SIMPLE = 0, 1
 OK = 0
+ENV_STATE_LOADED, ENV_STATE_BAD_ENV, ENV_STATE_INVALID = 0, 1, 2     # nav3d_load_envs status codes
 
 STATUS_NAMES = {0: "NAV3D_OK", -1: "NAV3D_ERR_INVALID", -2: "NAV3D_ERR_UNSUPPORTED", -3: "NAV3D_ERR_CUDA",
                 -4: "NAV3D_ERR_NOMEM", -5: "NAV3D_ERR_ROOM"}
@@ -72,6 +73,9 @@ SYMBOLS = {
     "nav3d_snapshot_bytes": (C.c_size_t, [_P]),
     "nav3d_snapshot": (C.c_int, [_P, _P, C.c_size_t]),
     "nav3d_restore": (C.c_int, [_P, _P, C.c_size_t]),
+    "nav3d_env_state_bytes": (C.c_size_t, [_P]),
+    "nav3d_save_envs": (C.c_int, [_P, _P, C.c_int32, _P, _P, _P]),
+    "nav3d_load_envs": (C.c_int, [_P, _P, C.c_int32, _P, _P, _P, _P]),
     "nav3d_sample_actions": (C.c_int, [_P, C.c_int32, C.c_int32, C.c_uint64, C.c_uint32, C.c_uint32, _P, C.c_int32, _P, _P, _P, _P]),
     "nav3d_gae": (C.c_int, [_P, _P, _P, _P, _P, C.c_float, C.c_float, C.c_int32, C.c_int32, _P, _P, _P]),
     "nav3d_lstm_prepare": (C.c_int, [_P]),

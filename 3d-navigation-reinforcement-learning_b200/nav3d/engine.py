@@ -212,6 +212,77 @@ class Engine:
         buf = np.ascontiguousarray(buf, dtype=np.uint8)
         check(self._lib.nav3d_restore(self._h, C.c_void_p(buf.ctypes.data), buf.size))
 
+    # ---- env-state blobs ---------------------------------------------------------------------------------------------
+    @property
+    def env_state_bytes(self) -> int:
+        """Bytes of one env-state blob (``nav3d_env_state_bytes``)."""
+        return int(self._lib.nav3d_env_state_bytes(self._h))
+
+    def _env_ids(self, env_ids) -> torch.Tensor:
+        """A list, range, numpy array, CPU or device tensor of env ids -> contiguous int32 [n] on the engine's device.  Ids
+        that do not fit int32 become -1 (out of range) instead of wrapping onto a valid env."""
+        t = env_ids if isinstance(env_ids, torch.Tensor) else torch.as_tensor(np.asarray(env_ids, dtype=np.int64))
+        if t.dim() != 1 or t.dtype.is_floating_point or t.dtype.is_complex or t.dtype == torch.bool:
+            raise ValueError(f"env_ids must be a 1-D integer sequence or tensor, got {t.dtype} {tuple(t.shape)}")
+        if t.dtype != torch.int32:
+            t = torch.where((t < 0) | (t >= self.n_envs), torch.full_like(t, -1), t)
+        return t.to(device=self.device, dtype=torch.int32).contiguous()
+
+    def save_envs(self, env_ids, obs: torch.Tensor, out: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """The complete state of the listed envs as uint8 [n, env_state_bytes] blobs on the engine's device.
+
+        ``obs`` is the observation array the last step / reset / load wrote: a blob carries its env's current row, which
+        cannot be recomputed from the env's record.  Asynchronous on the current stream; with a device tensor of ids and an
+        ``out`` buffer it can be captured in a CUDA graph.  An out-of-range id yields a blob every load rejects."""
+        ids = self._env_ids(env_ids)
+        n, B = ids.numel(), self.env_state_bytes
+        self._check(obs, torch.float32, (self.n_envs, self.obs_dim), "obs")
+        if out is None:
+            out = torch.empty((n, B), dtype=torch.uint8, device=self.device)
+        self._check(out, torch.uint8, (n, B), "out")
+        with torch.cuda.device(self.device):
+            check(self._lib.nav3d_save_envs(self._h, _ptr(ids), n, _ptr(obs), _ptr(out), self._stream()))
+        return out
+
+    def load_envs(self, env_ids, states: torch.Tensor, obs: torch.Tensor, *, check: bool = True) -> torch.Tensor:
+        """Overwrite the listed envs with ``states[i]`` (blobs from ``save_envs`` of this or an equally configured engine)
+        and write their observation rows into ``obs``, which is returned.  Cloning env ``a`` into envs ``dst``::
+
+            engine.load_envs(dst, engine.save_envs([a], obs)[[0] * len(dst)], obs)
+
+        ``check=True``: the ids must be in range and distinct (a ``Nav3dError`` otherwise, before anything is written), and
+        the per-blob status is read back after the launch (one synchronisation; device-tensor ids cost one more); a blob this
+        engine cannot load leaves its env untouched and raises a ``Nav3dError`` naming every bad entry.
+        ``check=False``: nothing synchronises (for use inside a captured CUDA graph); the ids must be distinct, and rejected
+        blobs leave their envs untouched silently."""
+        ids = self._env_ids(env_ids)
+        n, B = ids.numel(), self.env_state_bytes
+        self._check(states, torch.uint8, (n, B), "states")
+        self._check(obs, torch.float32, (self.n_envs, self.obs_dim), "obs")
+        status = None
+        if check:
+            h = ids.cpu().numpy()
+            bad = np.nonzero((h < 0) | (h >= self.n_envs))[0]
+            if len(bad):
+                raise Nav3dError(-1, f"load_envs: env ids out of range 0..{self.n_envs - 1} at entries "
+                                     f"{bad[:16].tolist()} (ids {h[bad[:16]].tolist()})")
+            uniq, counts = np.unique(h, return_counts=True)
+            if (counts > 1).any():
+                raise Nav3dError(-1, f"load_envs: env ids must be distinct; repeated: {uniq[counts > 1][:16].tolist()}")
+            status = torch.empty(n, dtype=torch.uint8, device=self.device)
+        with torch.cuda.device(self.device):
+            _lib.check(self._lib.nav3d_load_envs(self._h, _ptr(ids), n, _ptr(states), _ptr(obs), _ptr(status),
+                                                 self._stream()))
+        if check and n:
+            st = status.cpu().numpy()
+            bad = np.nonzero(st != _lib.ENV_STATE_LOADED)[0]
+            if len(bad):
+                raise Nav3dError(-1, f"load_envs: {len(bad)} of {n} blobs were not loaded (their envs are unchanged): "
+                                     + ", ".join(f"entry {i} -> env {int(h[i])}: "
+                                                 + ("env id out of range" if st[i] == _lib.ENV_STATE_BAD_ENV else
+                                                    "not a valid blob for this engine") for i in bad[:16]))
+        return obs
+
     @property
     def launch_count(self) -> int:
         return int(self._lib.nav3d_launch_count(self._h))

@@ -144,6 +144,17 @@ class BatchedCubicEnv:
     def state(self) -> torch.Tensor:
         return self.engine.get_state()
 
+    def save_envs(self, indices, obs: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """Complete state of the listed envs as uint8 [n, engine.env_state_bytes] device blobs (``Engine.save_envs``).
+        ``obs`` is the current observation array: this env's own buffer by default; pass the tensor the last
+        ``step_wait(out_obs=...)`` wrote when it was elsewhere."""
+        return self.engine.save_envs(indices, self._obs if obs is None else obs)
+
+    def load_envs(self, indices, states: torch.Tensor, obs: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """Overwrite the listed envs with blobs from ``save_envs`` and write their observation rows into ``obs`` (this env's
+        own buffer by default), which is returned.  Raises ``Nav3dError`` for bad ids or blobs (``Engine.load_envs``)."""
+        return self.engine.load_envs(indices, states, self._obs if obs is None else obs)
+
     def sb3_infos(self, info: StepInfo) -> List[dict]:
         return info.to_dicts(self._t_start)
 
@@ -242,6 +253,14 @@ class BatchedSimpleEnv:
     def step(self, actions):
         self.step_async(actions)
         return self.step_wait()
+
+    def save_envs(self, indices, obs: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """As ``BatchedCubicEnv.save_envs``."""
+        return self.engine.save_envs(indices, self._obs if obs is None else obs)
+
+    def load_envs(self, indices, states: torch.Tensor, obs: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """As ``BatchedCubicEnv.load_envs``."""
+        return self.engine.load_envs(indices, states, self._obs if obs is None else obs)
 
     def close(self):
         self.engine.close()

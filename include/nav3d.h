@@ -151,7 +151,8 @@ int nav3d_num_envs(const nav3d_engine *e);
 int nav3d_lanes_per_env(const nav3d_engine *e);
 
 /* GridAgent.reset (envs/CubicEnv.py:77-108) for a set of envs.
- *   env_ids : DEVICE int32[n] or NULL = envs 0..n-1 (then n must be <= n_envs)
+ *   env_ids : DEVICE int32[n] or NULL = envs 0..n-1 (then n must be <= n_envs); the listed ids must be distinct (two
+ *             resets of one env in one call race on its record and knowledge)
  *   picks   : DEVICE int32[n][2] = (room index, k-th free cell) per listed env — the two random.choice draws of
  *             load_room (:407, :462) — for a NAV3D_ENV_SIMPLE engine int32[n][3]: the third column is the index of the goal in the
  *             same free-cell list (envs/simpleEnv.py:419-426) — or NULL = draw them from the env's Philox reset stream.
@@ -202,6 +203,49 @@ int nav3d_get_grid(nav3d_engine *e, int32_t env, int16_t *grid, void *stream);
 size_t nav3d_snapshot_bytes(const nav3d_engine *e);
 int nav3d_snapshot(nav3d_engine *e, void *host_buf, size_t bytes);
 int nav3d_restore(nav3d_engine *e, const void *host_buf, size_t bytes);
+
+/* ---- env-state blobs: save the complete state of listed envs on the device and load it back, into the same envs or into
+ * others (ALE's cloneState / restoreState, per env).  Go-Explore-style archives, branching (one blob loaded into k envs),
+ * evaluation from fixed mid-episode states.
+ *
+ * A blob is nav3d_env_state_bytes bytes, 16-byte aligned, in caller-owned DEVICE memory; blob i of a call is at
+ * blobs + i * nav3d_env_state_bytes.  It holds a header (magic, format version, engine signature, room index, live byte
+ * counts), the env's 32-byte record (position, counters, episode number, return so far, ...), its observation row and its
+ * knowledge volume.  Only the live part of the knowledge is written — that of the env's current room — so a save of envs
+ * in small rooms moves little even in an engine sized for a large one; bytes past the live parts are left as they were.
+ * Blobs are plain bytes: they may be copied, duplicated, moved to another device or written to a file.
+ *
+ * The engine signature hashes the env kind, local_map_length, the per-env block size and the room table (each room's dims,
+ * wall code, grid and start position).  A blob loads into any engine with the same signature: lanes_per_env, seed, env_id0,
+ * n_envs, auto_reset and the reward parameters may differ.
+ *
+ * Observations: obs[68..70] of a CubicEnv row are the PREVIOUS step's last_action, was_near_wall and last_bump, which the
+ * record no longer holds, so the row cannot be recomputed from it.  nav3d_save_envs therefore copies each listed env's row
+ * out of `obs`, which must be the observation array the last nav3d_step / nav3d_reset / nav3d_load_envs wrote for that
+ * env, and nav3d_load_envs writes the row back.
+ *
+ * Semantics: a loaded env continues exactly as the saved env would have, with one exception: randomness stays keyed by
+ * the DESTINATION — its global id (env_id0 + index) and the engine seed — at the blob's episode counter.  Loading a blob
+ * back into the env it came from replays that env bit for bit, its later auto-resets included; a blob loaded into another
+ * env is identical until that env's next reset, which draws from the destination's Philox reset stream.
+ *
+ * Both calls are asynchronous on `stream`: no synchronisation, no allocation, no host copy, so they can be captured in a
+ * CUDA graph.  Both take env_ids = DEVICE int32[n] or NULL = envs 0..n-1 (then n <= n_envs). */
+
+/* Bytes of one env-state blob of this engine (fixed once rooms are loaded; 0 before). */
+size_t nav3d_env_state_bytes(const nav3d_engine *e);
+/* Copy the complete state of the listed envs into blobs[i] (DEVICE, n * nav3d_env_state_bytes).
+ *   obs : DEVICE f32[n_envs][obs_dim]: the caller's CURRENT observation of every env (required; see above)
+ * An env id outside 0..n_envs-1 gets a blob with an invalid magic, which every load rejects (status 2).  Env ids may
+ * repeat.  Fails with NAV3D_ERR_INVALID until the envs have been reset (or restored / loaded). */
+int nav3d_save_envs(nav3d_engine *e, const int32_t *env_ids, int32_t n, const float *obs, void *blobs, void *stream);
+/* Overwrite the listed envs with blobs[i] and write their observation rows into obs (DEVICE f32[n_envs][obs_dim]).
+ *   status : DEVICE u8[n] or NULL: 0 loaded, 1 env id out of range, 2 blob not valid for this engine (env untouched)
+ * Every blob's header (magic, version, signature, room index < n_rooms, live sizes) is checked before anything of its env
+ * is written.  The listed env ids must be distinct; blobs may repeat (loading one blob into many envs is the clone).
+ * Counts as a reset for the step-before-reset check, as nav3d_restore does. */
+int nav3d_load_envs(nav3d_engine *e, const int32_t *env_ids, int32_t n, const void *blobs, float *obs,
+                    uint8_t *status, void *stream);
 
 /* ---- rollout-loop kernels of the LSTM-PPO trainer (SURVEY §8f row 1).  Engine-free: they run on the CUDA device that is
  * current on the calling thread; all buffers are DEVICE pointers; asynchronous on `stream`.  They replace, in the
