@@ -903,6 +903,37 @@ NAV3D_HD bool step_env(const EngineParams &P, const StepIO &io, int env, int lan
     return c.will_reset;
 }
 
+// The [T][n_envs] arrays of one fused rollout (nav3d_rollout_actions; nav3d_rollout_random fills obs / obs_last / reward
+// only).  Any output may be null; with obs == null only the last step's rows are formed, into obs_last [n_envs][80].
+struct RolloutIO {
+    const uint8_t *actions;        // caller-supplied actions; values > 5 act as 5 (step_lane clamps)
+    float *obs, *obs_last, *reward;
+    double *reward64;
+    uint8_t *terminated, *truncated;
+    float *terminal_obs;
+    void *episodes;                // nav3d_episode*
+};
+
+// The StepIO of step t of a fused rollout: rows stay indexed by env, the row offsets are 64-bit ([32][2^20][80] f32 is
+// 10.7 GB).
+NAV3D_HD StepIO rollout_step_io(const RolloutIO &ro, int t, int T, long long n_envs) {
+    const long long r0 = (long long)t * n_envs;
+    StepIO io;
+    io.actions = nullptr;
+    io.obs = ro.obs ? ro.obs + r0 * kObsDim : (t == T - 1 ? ro.obs_last : nullptr);
+    io.reward = ro.reward ? ro.reward + r0 : nullptr;
+    io.reward64 = ro.reward64 ? ro.reward64 + r0 : nullptr;
+    io.terminated = ro.terminated ? ro.terminated + r0 : nullptr;
+    io.truncated = ro.truncated ? ro.truncated + r0 : nullptr;
+    io.terminal_obs = ro.terminal_obs ? ro.terminal_obs + r0 * kObsDim : nullptr;
+    io.episodes = ro.episodes ? static_cast<EpisodeRec *>(ro.episodes) + r0 : nullptr;
+    io.env0 = 0; io.env_n = (int)n_envs;
+    return io;
+}
+NAV3D_HD int rollout_action(const RolloutIO &ro, int t, long long n_envs, long long env) {
+    return ro.actions[(long long)t * n_envs + env];
+}
+
 // ===============================================================================================================
 // simpleEnv (envs/simpleEnv.py): ternary knowledge grid, ray-cell observations, goal reward
 //   step :109-150, do_action :152-186, compute_reward :189-217, get_obs :219-265, _mark_visited :273-298,

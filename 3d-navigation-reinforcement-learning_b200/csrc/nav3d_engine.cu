@@ -387,12 +387,15 @@ __global__ void __launch_bounds__(kBlock) reset_tpe_kernel(const __grid_constant
     tpe_reset<true>(P, mine, (uint32_t)env, episode, picks != nullptr, room, k, lut, obs, w, lane);
 }
 
-// T fused steps per env, thread per env (BASELINE.md §4 config 4: on-device Philox actions).  The record stays in the
-// thread's registers for the whole rollout and the knowledge lines it touches stay in L2, so DRAM sees the outputs the
-// caller asked for plus one pass over the touched lines.
-template <int BLOCK, bool STAGED>
+// T fused steps per env, thread per env.  The record stays in the thread's registers for the whole rollout and the
+// knowledge lines it touches stay in L2, so DRAM sees the outputs the caller asked for plus one pass over the touched lines.
+// CALLER_ACTIONS: the actions are the caller's u8 [T][N] rows (nav3d_rollout_actions) and every output of nav3d_step may
+// be written; otherwise they come from the env's Philox action stream (BASELINE.md §4 config 4: nav3d_rollout_random,
+// which also fills `done` and `actions_out`).  The Philox branches keep their own StepIO set-up: written through
+// rollout_step_io, nav3d_rollout_random compiled to different (if equivalent) SASS.
+template <int BLOCK, bool STAGED, bool CALLER_ACTIONS>
 __device__ __forceinline__ void rollout_tpe_body(const EngineParams &P, int T, uint32_t t0, float *obs, float *obs_last,
-                                                 float *reward, uint8_t *done, uint8_t *actions_out) {
+                                                 float *reward, uint8_t *done, uint8_t *actions_out, const RolloutIO *ro) {
     __shared__ float lut[kLutSize];
     __shared__ WarpWork work[STAGED ? BLOCK / 32 : 1];
     fill_lut(lut, P.L);
@@ -413,23 +416,34 @@ __device__ __forceinline__ void rollout_tpe_body(const EngineParams &P, int T, u
     if (valid) st = P.states[env];
     for (int t = 0; t < T; t++) {
         StepIO io;
-        io.actions = nullptr;
-        // obs == NULL: only the last step's observation is written out
-        io.obs = obs ? obs + (long long)t * N * kObsDim : (t == T - 1 ? obs_last : nullptr);
-        io.reward = reward ? reward + (long long)t * N : nullptr;
-        io.reward64 = nullptr; io.terminated = nullptr; io.truncated = nullptr;
-        io.terminal_obs = nullptr; io.episodes = nullptr;
-        io.env0 = 0; io.env_n = P.n_envs;
+        if constexpr (CALLER_ACTIONS) {
+            io = rollout_step_io(*ro, t, T, N);
+        } else {
+            io.actions = nullptr;
+            // obs == NULL: only the last step's observation is written out
+            io.obs = obs ? obs + (long long)t * N * kObsDim : (t == T - 1 ? obs_last : nullptr);
+            io.reward = reward ? reward + (long long)t * N : nullptr;
+            io.reward64 = nullptr; io.terminated = nullptr; io.truncated = nullptr;
+            io.terminal_obs = nullptr; io.episodes = nullptr;
+            io.env0 = 0; io.env_n = P.n_envs;
+        }
         if (STAGED) w->dst[lane] = nullptr;
         bool rst = false;
         if (valid) {
             uint32_t u0, u1, bits = 0;
-            philox4x32_10(P.env_id0 + (uint32_t)env, t0 + (uint32_t)t, 0u, kStreamAction, P.seed_lo, P.seed_hi, u0, u1);
-            const int action = (int)mulhi_range(u0, 6u);
+            int action;
+            if constexpr (CALLER_ACTIONS) {
+                action = rollout_action(*ro, t, N, env);
+            } else {
+                philox4x32_10(P.env_id0 + (uint32_t)env, t0 + (uint32_t)t, 0u, kStreamAction, P.seed_lo, P.seed_hi, u0, u1);
+                action = (int)mulhi_range(u0, 6u);
+            }
             rst = step_env<1, true, STAGED>(P, io, (int)env, 0, lane, action, lut, env, &st, &bits,
                                             w->stage + lane * kStageStride, w->dst + lane, STAGED ? &mq : nullptr);
-            if (done) done[(long long)t * N + env] = bits ? 1 : 0;
-            if (actions_out) actions_out[(long long)t * N + env] = (uint8_t)action;
+            if constexpr (!CALLER_ACTIONS) {
+                if (done) done[(long long)t * N + env] = bits ? 1 : 0;
+                if (actions_out) actions_out[(long long)t * N + env] = (uint8_t)action;
+            }
         }
         if (STAGED) coop_marks(P, w, lane, [&]() { flush_rows(w->stage, w->dst, lane, lut, P.L); });
         if (__any_sync(0xffffffffu, rst)) {
@@ -443,17 +457,21 @@ template <int BLOCK, int MINB, bool STAGED>
 __global__ void __launch_bounds__(BLOCK, MINB) rollout_tpe_kernel(const __grid_constant__ EngineParams P, int T, uint32_t t0,
                                                                   float *obs, float *obs_last, float *reward, uint8_t *done,
                                                                   uint8_t *actions_out) {
-    rollout_tpe_body<BLOCK, STAGED>(P, T, t0, obs, obs_last, reward, done, actions_out);
+    rollout_tpe_body<BLOCK, STAGED, false>(P, T, t0, obs, obs_last, reward, done, actions_out, nullptr);
 }
-// T fused steps per env with on-device Philox actions (SURVEY §8f row 3).  An env's record and the knowledge lines it
-// touches stay in L1/L2 for the whole rollout, so DRAM sees the outputs the caller asked for plus one pass over the touched
-// lines.  When only the last observation is requested the intermediate observations are never formed.  The reset is an
-// out-of-line call (as in step_call_kernel) so that the loop body keeps the step's 64 registers.
-template <int G, int MINB>
-__global__ void __launch_bounds__(kBlock, MINB) rollout_kernel(const __grid_constant__ EngineParams P, int T, uint32_t t0,
-                                                            float *obs, float *obs_last, float *reward, uint8_t *done,
-                                                            uint8_t *actions_out, float *reward_scratch,
-                                                            uint8_t *term_scratch, uint8_t *trunc_scratch) {
+template <int BLOCK, int MINB>
+__global__ void __launch_bounds__(BLOCK, MINB) rollout_actions_tpe_kernel(const __grid_constant__ EngineParams P, int T,
+                                                                          const __grid_constant__ RolloutIO ro) {
+    rollout_tpe_body<BLOCK, true, true>(P, T, 0u, nullptr, nullptr, nullptr, nullptr, nullptr, &ro);
+}
+// T fused steps per env, G lanes per env, actions as in rollout_tpe_body (SURVEY §8f row 3).  An env's record and the
+// knowledge lines it touches stay in L1/L2 for the whole rollout, so DRAM sees the outputs the caller asked for plus one
+// pass over the touched lines.  When only the last observation is requested the intermediate observations are never
+// formed.  The reset is an out-of-line call (as in step_call_kernel) so that the loop body keeps the step's 64 registers.
+template <int G, bool CALLER_ACTIONS>
+__device__ __forceinline__ void rollout_group_body(const EngineParams &P, int T, uint32_t t0, float *obs, float *obs_last,
+                                                   float *reward, uint8_t *done, uint8_t *actions_out,
+                                                   float *reward_scratch, const RolloutIO *ro) {
     __shared__ float lut[kLutSize];
     fill_lut(lut, P.L);
     const long long gid = (long long)blockIdx.x * kBlock + threadIdx.x;
@@ -464,17 +482,26 @@ __global__ void __launch_bounds__(kBlock, MINB) rollout_kernel(const __grid_cons
     EnvState st = P.states[env];          // the record stays in registers for the whole rollout (every lane holds a copy)
     for (int t = 0; t < T; t++) {
         uint32_t u0, u1;
-        philox4x32_10(P.env_id0 + (uint32_t)env, t0 + (uint32_t)t, 0u, kStreamAction, P.seed_lo, P.seed_hi, u0, u1);
-        const int action = (int)mulhi_range(u0, 6u);
+        int action;
+        if constexpr (CALLER_ACTIONS) {
+            action = rollout_action(*ro, t, N, env);
+        } else {
+            philox4x32_10(P.env_id0 + (uint32_t)env, t0 + (uint32_t)t, 0u, kStreamAction, P.seed_lo, P.seed_hi, u0, u1);
+            action = (int)mulhi_range(u0, 6u);
+        }
         StepIO io;
-        io.actions = nullptr;
-        // obs == NULL: only the last step's observation is kept; the earlier steps form none (and skip the window gather)
-        io.obs = obs ? obs + (long long)t * N * kObsDim : (t == T - 1 ? obs_last : nullptr);
-        io.reward = reward ? reward + (long long)t * N : reward_scratch;
-        io.reward64 = nullptr;
-        io.terminated = nullptr; io.truncated = nullptr;
-        io.terminal_obs = nullptr; io.episodes = nullptr;
-        io.env0 = 0; io.env_n = P.n_envs;
+        if constexpr (CALLER_ACTIONS) {
+            io = rollout_step_io(*ro, t, T, N);
+        } else {
+            io.actions = nullptr;
+            // obs == NULL: only the last step's observation is kept; the earlier steps form none (and skip the window gather)
+            io.obs = obs ? obs + (long long)t * N * kObsDim : (t == T - 1 ? obs_last : nullptr);
+            io.reward = reward ? reward + (long long)t * N : reward_scratch;
+            io.reward64 = nullptr;
+            io.terminated = nullptr; io.truncated = nullptr;
+            io.terminal_obs = nullptr; io.episodes = nullptr;
+            io.env0 = 0; io.env_n = P.n_envs;
+        }
         uint32_t bits = 0;
         if (step_env<G, true>(P, io, (int)env, lane, liw, action, lut, env, &st, &bits)) {
             group_sync<G>(liw);            // all lanes are done reading the old knowledge
@@ -482,13 +509,27 @@ __global__ void __launch_bounds__(kBlock, MINB) rollout_kernel(const __grid_cons
             group_sync<G>(liw);            // lane 0's record of the new episode is visible
             st = P.states[env];
         }
-        if (lane == 0) {
-            if (done) done[(long long)t * N + env] = bits ? 1 : 0;
-            if (actions_out) actions_out[(long long)t * N + env] = (uint8_t)action;
+        if constexpr (!CALLER_ACTIONS) {
+            if (lane == 0) {
+                if (done) done[(long long)t * N + env] = bits ? 1 : 0;
+                if (actions_out) actions_out[(long long)t * N + env] = (uint8_t)action;
+            }
         }
         group_sync<G>(liw);   // lane 0's counter store and every lane's S stores are visible to the next step
     }
     if (lane == 0) P.states[env] = st;
+}
+template <int G, int MINB>
+__global__ void __launch_bounds__(kBlock, MINB) rollout_kernel(const __grid_constant__ EngineParams P, int T, uint32_t t0,
+                                                            float *obs, float *obs_last, float *reward, uint8_t *done,
+                                                            uint8_t *actions_out, float *reward_scratch,
+                                                            uint8_t *term_scratch, uint8_t *trunc_scratch) {
+    rollout_group_body<G, false>(P, T, t0, obs, obs_last, reward, done, actions_out, reward_scratch, nullptr);
+}
+template <int G, int MINB>
+__global__ void __launch_bounds__(kBlock, MINB) rollout_actions_kernel(const __grid_constant__ EngineParams P, int T,
+                                                                    const __grid_constant__ RolloutIO ro) {
+    rollout_group_body<G, true>(P, T, 0u, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, &ro);
 }
 
 template <int G>
@@ -908,6 +949,7 @@ int nav3d_load_rooms(nav3d_engine *e, int32_t n_rooms, const nav3d_room_desc *ro
         if (pct > 0 && pct <= 100) {
             cudaFuncSetAttribute(step_tpe_kernel<64, 8, true>, cudaFuncAttributePreferredSharedMemoryCarveout, pct);
             cudaFuncSetAttribute(rollout_tpe_kernel<64, 8, true>, cudaFuncAttributePreferredSharedMemoryCarveout, pct);
+            cudaFuncSetAttribute(rollout_actions_tpe_kernel<64, 8>, cudaFuncAttributePreferredSharedMemoryCarveout, pct);
         }
     }
     size_t ovf_off = align_up(max_k, 128), stride = ovf_off + align_up(max_cells, 128);
@@ -1197,6 +1239,42 @@ int nav3d_rollout_random(nav3d_engine *e, int32_t T, uint32_t t0, float *obs, fl
         }
         rollout_kernel<G, 6><<<grid_for(e->cfg.n_envs, G), kBlock, 0, s>>>(e->P, T, t0, obs, obs_last, reward, done, actions_out,
                                                                            e->d_reward, e->d_term, e->d_trunc);
+        return NAV3D_OK;
+    });
+    if (rc) return rc;
+    e->launches++;
+    CUDA_TRY(cudaGetLastError());
+    return NAV3D_OK;
+}
+
+int nav3d_rollout_actions(nav3d_engine *e, int32_t T, const uint8_t *actions, float *obs, float *obs_last, float *reward,
+                          double *reward64, uint8_t *terminated, uint8_t *truncated, float *terminal_obs,
+                          nav3d_episode *episodes, void *stream) {
+    if (T < 0) return fail(NAV3D_ERR_INVALID, "T must be >= 0");
+    if (!actions) return fail(NAV3D_ERR_INVALID, "actions is required");
+    if (!obs && !obs_last) return fail(NAV3D_ERR_INVALID, "one of obs / obs_last is required");
+    if (((uintptr_t)obs | (uintptr_t)obs_last | (uintptr_t)terminal_obs) & 15u)
+        return fail(NAV3D_ERR_INVALID, "obs / obs_last / terminal_obs must be 16-byte aligned");
+    if (int rc = check_steppable(e)) return rc;
+    if (e->simple) return fail(NAV3D_ERR_UNSUPPORTED, "nav3d_rollout_actions is implemented for NAV3D_ENV_CUBIC only");
+    if (T == 0) return NAV3D_OK;
+    NAV3D_DEVICE(e);
+    NvtxRange range("nav3d_rollout_actions");
+    RolloutIO ro;
+    ro.actions = actions; ro.obs = obs; ro.obs_last = obs_last; ro.reward = reward; ro.reward64 = reward64;
+    ro.terminated = terminated; ro.truncated = truncated; ro.terminal_obs = terminal_obs; ro.episodes = episodes;
+    cudaStream_t s = (cudaStream_t)stream;
+    const int n = e->cfg.n_envs;
+    int rc = dispatch_lanes(e->G, [&](auto g) {
+        constexpr int G = decltype(g)::value;
+        if constexpr (G == 1) {           // the launch configurations of nav3d_rollout_random
+            const size_t smem = (size_t)(e->tpe_block / 32) * e->P.mark_cap * sizeof(uint32_t);
+            if (e->tpe_block == 64) rollout_actions_tpe_kernel<64, 8><<<(unsigned)((n + 63) / 64), 64, smem, s>>>(e->P, T, ro);
+            else if (e->minb == 4) rollout_actions_tpe_kernel<128, 4><<<grid_for(n, 1), kBlock, smem, s>>>(e->P, T, ro);
+            else rollout_actions_tpe_kernel<128, 3><<<grid_for(n, 1), kBlock, smem, s>>>(e->P, T, ro);
+        } else {
+            rollout_actions_kernel<G, 6><<<grid_for(n, G), kBlock, 0, s>>>(e->P, T, ro);
+        }
         return NAV3D_OK;
     });
     if (rc) return rc;

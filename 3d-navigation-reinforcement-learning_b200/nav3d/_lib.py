@@ -68,6 +68,7 @@ SYMBOLS = {
     "nav3d_step": (C.c_int, [_P, _P, _P, _P, _P, _P, _P, _P, _P, _P]),
     "nav3d_step_host": (C.c_int, [_P, _P, _P, _P, _P, _P]),
     "nav3d_rollout_random": (C.c_int, [_P, C.c_int32, C.c_uint32, _P, _P, _P, _P, _P, _P]),
+    "nav3d_rollout_actions": (C.c_int, [_P, C.c_int32] + [_P] * 10),
     "nav3d_get_state": (C.c_int, [_P, _P, _P]),
     "nav3d_get_grid": (C.c_int, [_P, C.c_int32, _P, _P]),
     "nav3d_snapshot_bytes": (C.c_size_t, [_P]),

@@ -185,6 +185,47 @@ class Engine:
             check(self._lib.nav3d_rollout_random(self._h, int(T), int(t0) & 0xFFFFFFFF, _ptr(obs), _ptr(obs_last),
                                                  _ptr(reward), _ptr(done), _ptr(actions_out), self._stream()))
 
+    def rollout_actions(self, actions: torch.Tensor, *, obs: Optional[torch.Tensor] = None,
+                        obs_last: Optional[torch.Tensor] = None, reward: Optional[torch.Tensor] = None,
+                        reward64: Optional[torch.Tensor] = None, terminated: Optional[torch.Tensor] = None,
+                        truncated: Optional[torch.Tensor] = None, terminal_obs: Optional[torch.Tensor] = None,
+                        episodes: Optional[torch.Tensor] = None):
+        """T steps of every env with the rows of ``actions`` [T, n_envs] in one fused launch (``nav3d_rollout_actions``):
+        every output and the final engine state equal those of T ``step`` calls with the same rows.
+
+        ``actions``: uint8 on the engine's device is passed as it is (``rollout_random``'s ``actions_out`` replays as it
+        is); any other integer dtype is clamped to 0..5 and cast, which is what ``step`` does to int64.  The outputs are
+        ``step``'s with a leading T axis, all optional; ``obs_last`` [n_envs, obs_dim] receives the last step's rows when
+        ``obs`` is None, and one of the two is required.  Rows of ``terminal_obs`` and ``episodes`` are written only where
+        an episode ended.  Asynchronous on the current stream; with uint8 actions it allocates nothing and can be captured
+        in a CUDA graph."""
+        if (not isinstance(actions, torch.Tensor) or actions.dim() != 2 or actions.dtype.is_floating_point
+                or actions.dtype.is_complex or actions.dtype == torch.bool):
+            raise ValueError(f"actions must be a 2-D integer tensor [T, {self.n_envs}], got "
+                             f"{getattr(actions, 'dtype', type(actions))} {tuple(getattr(actions, 'shape', ()))}")
+        T, N = int(actions.shape[0]), self.n_envs
+        if actions.dtype != torch.uint8:
+            actions = actions.to(self.device).clamp(0, 5).to(torch.uint8).contiguous()
+        self._check(actions, torch.uint8, (T, N), "actions")
+        for t, dtype, shape, name in ((obs, torch.float32, (T, N, self.obs_dim), "obs"),
+                                      (obs_last, torch.float32, (N, self.obs_dim), "obs_last"),
+                                      (reward, torch.float32, (T, N), "reward"),
+                                      (reward64, torch.float64, (T, N), "reward64"),
+                                      (terminated, torch.uint8, (T, N), "terminated"),
+                                      (truncated, torch.uint8, (T, N), "truncated"),
+                                      (terminal_obs, torch.float32, (T, N, self.obs_dim), "terminal_obs"),
+                                      (episodes, torch.int32, (T, N, 8), "episodes")):
+            if t is not None:
+                self._check(t, dtype, shape, name)
+        if obs is None and obs_last is None:
+            raise ValueError("one of obs / obs_last is required")
+        if T == 0:                     # (the buffers of an empty rollout have no storage to pass)
+            return
+        with torch.cuda.device(self.device):
+            check(self._lib.nav3d_rollout_actions(self._h, T, _ptr(actions), _ptr(obs), _ptr(obs_last), _ptr(reward),
+                                                  _ptr(reward64), _ptr(terminated), _ptr(truncated), _ptr(terminal_obs),
+                                                  _ptr(episodes), self._stream()))
+
     # ---- state -------------------------------------------------------------------------------------------------
     def get_state(self) -> torch.Tensor:
         """int32 [n_envs, 16]; columns are ``STATE_FIELDS``."""

@@ -29,6 +29,10 @@ class StepInfo:
     terminal_observation: torch.Tensor  # f32 [N, 80]; rows valid where done
     episodes: torch.Tensor              # int32 [N, 8] view of nav3d_episode; rows valid where done
 
+    def __getitem__(self, t) -> "StepInfo":
+        """Step t of the per-step tensors ``BatchedCubicEnv.step_sequence`` returns (they carry a leading T axis)."""
+        return StepInfo(self.terminated[t], self.truncated[t], self.terminal_observation[t], self.episodes[t])
+
     def to_dicts(self, t_start: Optional[float] = None) -> List[dict]:
         term = self.terminated.cpu().numpy().astype(bool)
         trunc = self.truncated.cpu().numpy().astype(bool)
@@ -107,6 +111,30 @@ class BatchedCubicEnv:
 
     def seed(self, seed: Optional[int] = None):
         return [None] * self.num_envs
+
+    def step_sequence(self, actions):
+        """T calls of ``step()`` with the rows of ``actions`` [T, num_envs] in one fused launch (``Engine.rollout_actions``).
+
+        Returns ``obs`` [T, N, 80], ``rewards`` [T, N], ``dones`` [T, N] (bool) and a ``StepInfo`` whose tensors carry the
+        same leading T axis; ``info[t]`` is step t's (``sb3_infos(info[t])`` renders it).  Rows of terminal_observation and
+        episodes are valid where ``dones``.  The env's own observation buffer is left equal to ``obs[-1]``, so ``step()``,
+        ``save_envs()`` and ``step_sequence()`` continue from there."""
+        a = torch.as_tensor(actions)
+        if a.dim() != 2 or a.shape[1] != self.num_envs:
+            raise ValueError(f"actions must have shape (T, {self.num_envs}), got {tuple(a.shape)}")
+        a = a.to(self.device)
+        T, N, dev = int(a.shape[0]), self.num_envs, self.device
+        obs = torch.empty((T, N, 80), dtype=torch.float32, device=dev)
+        rewards = torch.empty((T, N), dtype=torch.float32, device=dev)
+        term = torch.empty((T, N), dtype=torch.uint8, device=dev)
+        trunc = torch.empty((T, N), dtype=torch.uint8, device=dev)
+        tobs = torch.zeros((T, N, 80), dtype=torch.float32, device=dev)
+        eps = torch.zeros((T, N, 8), dtype=torch.int32, device=dev)
+        self.engine.rollout_actions(a, obs=obs, reward=rewards, terminated=term, truncated=trunc, terminal_obs=tobs,
+                                    episodes=eps)
+        if T:
+            self._obs.copy_(obs[-1])
+        return obs, rewards, (term | trunc).bool(), StepInfo(term, trunc, tobs, eps)
 
     def close(self) -> None:
         self.engine.close()

@@ -189,6 +189,25 @@ int nav3d_step_host(nav3d_engine *e, const int64_t *actions, float *obs, float *
 int nav3d_rollout_random(nav3d_engine *e, int32_t T, uint32_t t0, float *obs, float *obs_last, float *reward,
                          uint8_t *done, uint8_t *actions_out, void *stream);
 
+/* T fused steps of every env with CALLER-SUPPLIED actions: the same work, outputs and auto-resets as T successive
+ * nav3d_step calls with the rows of `actions`, in one launch (record in registers, knowledge lines on chip across steps).
+ * Every byte it writes, and the engine state it leaves (nav3d_get_state, nav3d_get_grid, nav3d_save_envs blobs), equal
+ * those of the T nav3d_step calls; rows those calls would leave untouched are left untouched.
+ *   actions      : DEVICE u8[T][n_envs] (required); values > 5 act as 5, as nav3d_step clamps.  nav3d_rollout_random's
+ *                  actions_out is in this format, so a random rollout can be replayed as it is.
+ *   obs          : DEVICE f32[T][n_envs][80] or NULL;  obs_last : DEVICE f32[n_envs][80] or NULL (one of them required;
+ *                  with obs == NULL only the last step's rows are formed, as in nav3d_rollout_random)
+ *   reward       : DEVICE f32[T][n_envs] or NULL;   reward64 : DEVICE f64[T][n_envs] or NULL
+ *   terminated, truncated : DEVICE u8[T][n_envs] or NULL
+ *   terminal_obs : DEVICE f32[T][n_envs][80] or NULL; row [t][i] written only if env i auto-reset in step t
+ *   episodes     : DEVICE nav3d_episode[T][n_envs] or NULL; row [t][i] written only if env i's episode ended in step t
+ * obs / obs_last / terminal_obs 16-byte aligned.  CubicEnv only (NAV3D_ERR_UNSUPPORTED for simpleEnv, as
+ * nav3d_rollout_random).  The arguments are checked in this order before the engine is: T >= 0, actions, obs / obs_last,
+ * alignment.  T == 0 does nothing.  Asynchronous, no allocation, no synchronisation: capturable in a CUDA graph. */
+int nav3d_rollout_actions(nav3d_engine *e, int32_t T, const uint8_t *actions, float *obs, float *obs_last,
+                          float *reward, double *reward64, uint8_t *terminated, uint8_t *truncated,
+                          float *terminal_obs, nav3d_episode *episodes, void *stream);
+
 /* Integer state of every env (attributes read by the reference's callers: get_position CubicEnv.py:399-400,
  * visited_count/bump_count/done evaluate_grid.py:216-218, ...).  DEVICE int32[n_envs][NAV3D_STATE_INTS]:
  *  0 x  1 y  2 z  3 facing  4 visited_count  5 bump_count  6 step_count  7 near_wall  8 was_near_wall  9 last_bump
