@@ -27,8 +27,9 @@
 //   * G = 1 with STAGED (the default kernels of nav3d_engine.cu): one thread owns an env; its observation row leaves in
 //     compact form through a shared-memory staging tile that the warp expands and writes out, and its ray marking is
 //     queued for the warp (MarkQueue) instead of being done in the thread;
-//   * G = 2 .. 32 lanes per env (and G = 1 without STAGED): the lanes split the window columns and the marking tiles, each
-//     lane streams its own float4s; the only cross-lane traffic is one OR-reduction of the neighbour codes.
+//   * G = 2 .. 32 lanes per env (and G = 1 without STAGED, as the host emulation runs it): the lanes split the window
+//     columns and the marking tiles, each lane streams its own float4s; the only cross-lane traffic is one OR-reduction of
+//     the neighbour codes.
 #pragma once
 #include <stdint.h>
 #include <cuda_runtime.h>
@@ -904,7 +905,8 @@ NAV3D_HD bool step_env(const EngineParams &P, const StepIO &io, int env, int lan
 }
 
 // The [T][n_envs] arrays of one fused rollout (nav3d_rollout_actions; nav3d_rollout_random fills obs / obs_last / reward
-// only).  Any output may be null; with obs == null only the last step's rows are formed, into obs_last [n_envs][80].
+// and its own done / actions_out / t0, and leaves the rest null).  Any output may be null; with obs == null only the last
+// step's rows are formed, into obs_last [n_envs][80].
 struct RolloutIO {
     const uint8_t *actions;        // caller-supplied actions; values > 5 act as 5 (step_lane clamps)
     float *obs, *obs_last, *reward;
@@ -912,6 +914,8 @@ struct RolloutIO {
     uint8_t *terminated, *truncated;
     float *terminal_obs;
     void *episodes;                // nav3d_episode*
+    uint8_t *done, *actions_out;   // Philox actions: terminated | truncated, and the actions played
+    uint32_t t0;                   // Philox actions: step index of the first step in the env's action stream
 };
 
 // The StepIO of step t of a fused rollout: rows stay indexed by env, the row offsets are 64-bit ([32][2^20][80] f32 is

@@ -8,7 +8,6 @@
 
 #include <algorithm>
 #include <cstdio>
-#include <cstdlib>
 #include <cmath>
 #include <cstring>
 #include <string>
@@ -154,10 +153,10 @@ __device__ __noinline__ void reset_out_of_line(const EngineParams &P, int env, i
     reset_env_philox<G>(P, env, lane, liw, episode, lut, obs_row);
 }
 
-template <int G, int MINB>
-__global__ void __launch_bounds__(kBlock, MINB) step_call_kernel(const __grid_constant__ EngineParams P, StepIO io) {
+template <int G>
+__global__ void __launch_bounds__(kBlock, 8) step_call_kernel(const __grid_constant__ EngineParams P, StepIO io) {
     __shared__ float lut[kLutSize];
-    // Programmatic dependent launch: when launched with the stream-serialisation attribute this grid may become resident
+    // Programmatic dependent launch: launch_step sets the stream-serialisation attribute, so this grid may become resident
     // while the previous kernel of the stream is still draining; everything up to the wait (table fill, index math) overlaps
     // that tail, and the next kernel is allowed to do the same with ours.  Without the attribute both are no-ops.
     asm volatile("griddepcontrol.launch_dependents;");
@@ -179,7 +178,11 @@ __global__ void __launch_bounds__(kBlock, MINB) step_call_kernel(const __grid_co
 // Thread-per-env kernels (CubicEnv, lanes_per_env = 1): nothing of a step is computed twice, every load of a step is issued
 // by the one thread that needs it, and the only cooperation is in data movement — the warp writes the 32 observation rows
 // it assembled in shared memory with coalesced 128-bit stores, and clears the knowledge of the envs it resets together.
+// The step and rollout kernels run 64-thread CTAs, 8 per SM (128 registers, 16 warps per SM): the sweeps of DESIGN.md
+// §4 / §6.
 // ---------------------------------------------------------------------------------------------------------------
+constexpr int kTpeBlock = 64, kTpeMinBlocks = 8;
+
 // The warp's 32 staged (compact) rows -> their global rows (dst[e] == NULL: env e has none): get_obs Steps 2-6
 // (CubicEnv.py:270-307) — clip to [-2, 20] and (m + 2) / 22 through the code table, facing one-hot, the scalar quotients,
 // zero padding.  Two passes so that every store instruction runs ONE code path: the 16 window float4 of two envs per
@@ -297,7 +300,6 @@ __device__ __forceinline__ void coop_marks(const EngineParams &P, WarpWork *w, i
 
 // Auto-reset of the warp's envs whose lanes say `mine` (CubicEnv.py:77-108 with Philox picks).  Out of line so that the
 // step keeps its registers.  The new record goes to P.states.
-template <bool STAGED>
 __device__ __noinline__ void tpe_reset(const EngineParams &P, bool mine, uint32_t env, uint32_t episode, bool have_picks,
                                        uint32_t room, uint32_t k, const float *lut, float *obs, WarpWork *w, int lane) {
     const unsigned rmask = __ballot_sync(0xffffffffu, mine);
@@ -312,51 +314,44 @@ __device__ __noinline__ void tpe_reset(const EngineParams &P, bool mine, uint32_
         for (uint32_t i = (uint32_t)lane; i < n; i += 32u) k4[i] = zero;
     }
     __syncwarp();
-    if (STAGED) w->dst[lane] = nullptr;
+    w->dst[lane] = nullptr;
     if (mine) {
         ResetCtx c;
         float *row = obs ? obs + (unsigned long long)env * kObsDim : nullptr;
         MarkQueue mq{w->tasks, &w->n_tasks, w->desc, lane};
-        if (STAGED) { w->dst[lane] = row; if (row) row = w->stage + lane * kStageStride; }
-        const uint32_t nbr = reset_lane<1, STAGED>(P, (int)env, 0, room, k, episode + 1u, lut, row, c, STAGED ? &mq : nullptr);
+        w->dst[lane] = row; if (row) row = w->stage + lane * kStageStride;
+        const uint32_t nbr = reset_lane<1, true>(P, (int)env, 0, room, k, episode + 1u, lut, row, c, &mq);
         reset_commit(P, (int)env, 0, c, nbr);
     }
-    if (STAGED) coop_marks(P, w, lane, [&]() { flush_rows(w->stage, w->dst, lane, lut, P.L); });
+    coop_marks(P, w, lane, [&]() { flush_rows(w->stage, w->dst, lane, lut, P.L); });
 }
 
-template <int BLOCK, bool STAGED>
-__device__ __forceinline__ void step_tpe_body(const EngineParams &P, const StepIO &io) {
+__global__ void __launch_bounds__(kTpeBlock, kTpeMinBlocks) step_tpe_kernel(const __grid_constant__ EngineParams P, StepIO io) {
     __shared__ float lut[kLutSize];
-    __shared__ WarpWork work[STAGED ? BLOCK / 32 : 1];
+    __shared__ WarpWork work[kTpeBlock / 32];
     asm volatile("griddepcontrol.launch_dependents;");          // programmatic dependent launch, as in step_call_kernel
     fill_lut(lut, P.L);
     asm volatile("griddepcontrol.wait;" ::: "memory");
     const int lane = threadIdx.x & 31;
-    WarpWork *w = work + (STAGED ? threadIdx.x >> 5 : 0);
-    const long long gid = (long long)blockIdx.x * BLOCK + threadIdx.x;
+    WarpWork *w = work + (threadIdx.x >> 5);
+    const long long gid = (long long)blockIdx.x * kTpeBlock + threadIdx.x;
     if (gid - lane >= io.env_n) return;                          // the whole warp is past the range
     const bool valid = gid < io.env_n;
     const long long env = io.env0 + gid;
-    if (STAGED) {
-        w->dst[lane] = nullptr; w->env_of_lane[lane] = (uint32_t)env;
-        if (lane == 0) { w->n_tasks = 0; w->tasks = warp_tasks(P); }
-        __syncwarp();
-    }
+    w->dst[lane] = nullptr; w->env_of_lane[lane] = (uint32_t)env;
+    if (lane == 0) { w->n_tasks = 0; w->tasks = warp_tasks(P); }
+    __syncwarp();
     bool rst = false;
     if (valid) {
         MarkQueue mq{w->tasks, &w->n_tasks, w->desc, lane};
-        rst = step_env<1, false, STAGED>(P, io, (int)env, 0, lane, (int)io.actions[env], lut, env, nullptr, nullptr,
-                                         w->stage + lane * kStageStride, w->dst + lane, STAGED ? &mq : nullptr);
+        rst = step_env<1, false, true>(P, io, (int)env, 0, lane, (int)io.actions[env], lut, env, nullptr, nullptr,
+                                       w->stage + lane * kStageStride, w->dst + lane, &mq);
     }
-    if (STAGED) coop_marks(P, w, lane, [&]() { flush_rows(w->stage, w->dst, lane, lut, P.L); });
+    coop_marks(P, w, lane, [&]() { flush_rows(w->stage, w->dst, lane, lut, P.L); });
     if (__any_sync(0xffffffffu, rst)) {
         const uint32_t episode = rst ? P.states[env].episode : 0u;   // untouched by a step that ends its episode
-        tpe_reset<STAGED>(P, rst, (uint32_t)env, episode, false, 0u, 0u, lut, io.obs, w, lane);
+        tpe_reset(P, rst, (uint32_t)env, episode, false, 0u, 0u, lut, io.obs, w, lane);
     }
-}
-template <int BLOCK, int MINB, bool STAGED>
-__global__ void __launch_bounds__(BLOCK, MINB) step_tpe_kernel(const __grid_constant__ EngineParams P, StepIO io) {
-    step_tpe_body<BLOCK, STAGED>(P, io);
 }
 __global__ void __launch_bounds__(kBlock) reset_tpe_kernel(const __grid_constant__ EngineParams P,
                                                            const int32_t *__restrict__ env_ids, int n,
@@ -384,94 +379,74 @@ __global__ void __launch_bounds__(kBlock) reset_tpe_kernel(const __grid_constant
     w->env_of_lane[lane] = mine ? (uint32_t)env : 0u;
     if (lane == 0) { w->n_tasks = 0; w->tasks = warp_tasks(P); }
     __syncwarp();
-    tpe_reset<true>(P, mine, (uint32_t)env, episode, picks != nullptr, room, k, lut, obs, w, lane);
+    tpe_reset(P, mine, (uint32_t)env, episode, picks != nullptr, room, k, lut, obs, w, lane);
 }
 
+// nav3d_rollout_random writes obs / obs_last / reward only.  Its other per-step outputs are made null at compile time, so
+// the step drops their tests; tested at run time they cost the Philox rollout about 2 % (B200).
+__device__ __forceinline__ RolloutIO random_outputs(const RolloutIO &ro) {
+    RolloutIO r{};
+    r.obs = ro.obs; r.obs_last = ro.obs_last; r.reward = ro.reward;
+    return r;
+}
 // T fused steps per env, thread per env.  The record stays in the thread's registers for the whole rollout and the
 // knowledge lines it touches stay in L2, so DRAM sees the outputs the caller asked for plus one pass over the touched lines.
-// CALLER_ACTIONS: the actions are the caller's u8 [T][N] rows (nav3d_rollout_actions) and every output of nav3d_step may
-// be written; otherwise they come from the env's Philox action stream (BASELINE.md §4 config 4: nav3d_rollout_random,
-// which also fills `done` and `actions_out`).  The Philox branches keep their own StepIO set-up: written through
-// rollout_step_io, nav3d_rollout_random compiled to different (if equivalent) SASS.
-template <int BLOCK, bool STAGED, bool CALLER_ACTIONS>
-__device__ __forceinline__ void rollout_tpe_body(const EngineParams &P, int T, uint32_t t0, float *obs, float *obs_last,
-                                                 float *reward, uint8_t *done, uint8_t *actions_out, const RolloutIO *ro) {
+// CALLER_ACTIONS: the actions are the caller's u8 [T][N] rows (nav3d_rollout_actions); otherwise they come from the env's
+// Philox action stream (BASELINE.md §4 config 4: nav3d_rollout_random, which also fills `done` and `actions_out`).
+template <bool CALLER_ACTIONS>
+__global__ void __launch_bounds__(kTpeBlock, kTpeMinBlocks) rollout_tpe_kernel(const __grid_constant__ EngineParams P, int T,
+                                                                            const __grid_constant__ RolloutIO ro) {
     __shared__ float lut[kLutSize];
-    __shared__ WarpWork work[STAGED ? BLOCK / 32 : 1];
+    __shared__ WarpWork work[kTpeBlock / 32];
     fill_lut(lut, P.L);
     const int lane = threadIdx.x & 31;
-    WarpWork *w = work + (STAGED ? threadIdx.x >> 5 : 0);
-    const long long gid = (long long)blockIdx.x * BLOCK + threadIdx.x;
+    WarpWork *w = work + (threadIdx.x >> 5);
+    const long long gid = (long long)blockIdx.x * kTpeBlock + threadIdx.x;
     const long long N = P.n_envs;
     if (gid - lane >= N) return;
     const bool valid = gid < N;
     const long long env = gid;
-    if (STAGED) {
-        w->env_of_lane[lane] = (uint32_t)env;
-        if (lane == 0) { w->n_tasks = 0; w->tasks = warp_tasks(P); }
-        __syncwarp();
-    }
+    w->env_of_lane[lane] = (uint32_t)env;
+    if (lane == 0) { w->n_tasks = 0; w->tasks = warp_tasks(P); }
+    __syncwarp();
     const MarkQueue mq{w->tasks, &w->n_tasks, w->desc, lane};
     EnvState st;
     if (valid) st = P.states[env];
     for (int t = 0; t < T; t++) {
-        StepIO io;
-        if constexpr (CALLER_ACTIONS) {
-            io = rollout_step_io(*ro, t, T, N);
-        } else {
-            io.actions = nullptr;
-            // obs == NULL: only the last step's observation is written out
-            io.obs = obs ? obs + (long long)t * N * kObsDim : (t == T - 1 ? obs_last : nullptr);
-            io.reward = reward ? reward + (long long)t * N : nullptr;
-            io.reward64 = nullptr; io.terminated = nullptr; io.truncated = nullptr;
-            io.terminal_obs = nullptr; io.episodes = nullptr;
-            io.env0 = 0; io.env_n = P.n_envs;
-        }
-        if (STAGED) w->dst[lane] = nullptr;
+        const StepIO io = CALLER_ACTIONS ? rollout_step_io(ro, t, T, N) : rollout_step_io(random_outputs(ro), t, T, N);
+        w->dst[lane] = nullptr;
         bool rst = false;
         if (valid) {
             uint32_t u0, u1, bits = 0;
             int action;
             if constexpr (CALLER_ACTIONS) {
-                action = rollout_action(*ro, t, N, env);
+                action = rollout_action(ro, t, N, env);
             } else {
-                philox4x32_10(P.env_id0 + (uint32_t)env, t0 + (uint32_t)t, 0u, kStreamAction, P.seed_lo, P.seed_hi, u0, u1);
+                philox4x32_10(P.env_id0 + (uint32_t)env, ro.t0 + (uint32_t)t, 0u, kStreamAction, P.seed_lo, P.seed_hi, u0, u1);
                 action = (int)mulhi_range(u0, 6u);
             }
-            rst = step_env<1, true, STAGED>(P, io, (int)env, 0, lane, action, lut, env, &st, &bits,
-                                            w->stage + lane * kStageStride, w->dst + lane, STAGED ? &mq : nullptr);
+            rst = step_env<1, true, true>(P, io, (int)env, 0, lane, action, lut, env, &st, &bits,
+                                          w->stage + lane * kStageStride, w->dst + lane, &mq);
             if constexpr (!CALLER_ACTIONS) {
-                if (done) done[(long long)t * N + env] = bits ? 1 : 0;
-                if (actions_out) actions_out[(long long)t * N + env] = (uint8_t)action;
+                if (ro.done) ro.done[(long long)t * N + env] = bits ? 1 : 0;
+                if (ro.actions_out) ro.actions_out[(long long)t * N + env] = (uint8_t)action;
             }
         }
-        if (STAGED) coop_marks(P, w, lane, [&]() { flush_rows(w->stage, w->dst, lane, lut, P.L); });
+        coop_marks(P, w, lane, [&]() { flush_rows(w->stage, w->dst, lane, lut, P.L); });
         if (__any_sync(0xffffffffu, rst)) {
-            tpe_reset<STAGED>(P, rst, (uint32_t)env, st.episode, false, 0u, 0u, lut, io.obs, w, lane);
+            tpe_reset(P, rst, (uint32_t)env, st.episode, false, 0u, 0u, lut, io.obs, w, lane);
             if (rst) st = P.states[env];           // the new episode's record (written by this very thread)
         }
     }
     if (valid) P.states[env] = st;
 }
-template <int BLOCK, int MINB, bool STAGED>
-__global__ void __launch_bounds__(BLOCK, MINB) rollout_tpe_kernel(const __grid_constant__ EngineParams P, int T, uint32_t t0,
-                                                                  float *obs, float *obs_last, float *reward, uint8_t *done,
-                                                                  uint8_t *actions_out) {
-    rollout_tpe_body<BLOCK, STAGED, false>(P, T, t0, obs, obs_last, reward, done, actions_out, nullptr);
-}
-template <int BLOCK, int MINB>
-__global__ void __launch_bounds__(BLOCK, MINB) rollout_actions_tpe_kernel(const __grid_constant__ EngineParams P, int T,
-                                                                          const __grid_constant__ RolloutIO ro) {
-    rollout_tpe_body<BLOCK, true, true>(P, T, 0u, nullptr, nullptr, nullptr, nullptr, nullptr, &ro);
-}
-// T fused steps per env, G lanes per env, actions as in rollout_tpe_body (SURVEY §8f row 3).  An env's record and the
+// T fused steps per env, G lanes per env, actions as in rollout_tpe_kernel (SURVEY §8f row 3).  An env's record and the
 // knowledge lines it touches stay in L1/L2 for the whole rollout, so DRAM sees the outputs the caller asked for plus one
 // pass over the touched lines.  When only the last observation is requested the intermediate observations are never
 // formed.  The reset is an out-of-line call (as in step_call_kernel) so that the loop body keeps the step's 64 registers.
 template <int G, bool CALLER_ACTIONS>
-__device__ __forceinline__ void rollout_group_body(const EngineParams &P, int T, uint32_t t0, float *obs, float *obs_last,
-                                                   float *reward, uint8_t *done, uint8_t *actions_out,
-                                                   float *reward_scratch, const RolloutIO *ro) {
+__global__ void __launch_bounds__(kBlock, 6) rollout_kernel(const __grid_constant__ EngineParams P, int T,
+                                                            const __grid_constant__ RolloutIO ro) {
     __shared__ float lut[kLutSize];
     fill_lut(lut, P.L);
     const long long gid = (long long)blockIdx.x * kBlock + threadIdx.x;
@@ -484,24 +459,12 @@ __device__ __forceinline__ void rollout_group_body(const EngineParams &P, int T,
         uint32_t u0, u1;
         int action;
         if constexpr (CALLER_ACTIONS) {
-            action = rollout_action(*ro, t, N, env);
+            action = rollout_action(ro, t, N, env);
         } else {
-            philox4x32_10(P.env_id0 + (uint32_t)env, t0 + (uint32_t)t, 0u, kStreamAction, P.seed_lo, P.seed_hi, u0, u1);
+            philox4x32_10(P.env_id0 + (uint32_t)env, ro.t0 + (uint32_t)t, 0u, kStreamAction, P.seed_lo, P.seed_hi, u0, u1);
             action = (int)mulhi_range(u0, 6u);
         }
-        StepIO io;
-        if constexpr (CALLER_ACTIONS) {
-            io = rollout_step_io(*ro, t, T, N);
-        } else {
-            io.actions = nullptr;
-            // obs == NULL: only the last step's observation is kept; the earlier steps form none (and skip the window gather)
-            io.obs = obs ? obs + (long long)t * N * kObsDim : (t == T - 1 ? obs_last : nullptr);
-            io.reward = reward ? reward + (long long)t * N : reward_scratch;
-            io.reward64 = nullptr;
-            io.terminated = nullptr; io.truncated = nullptr;
-            io.terminal_obs = nullptr; io.episodes = nullptr;
-            io.env0 = 0; io.env_n = P.n_envs;
-        }
+        const StepIO io = CALLER_ACTIONS ? rollout_step_io(ro, t, T, N) : rollout_step_io(random_outputs(ro), t, T, N);
         uint32_t bits = 0;
         if (step_env<G, true>(P, io, (int)env, lane, liw, action, lut, env, &st, &bits)) {
             group_sync<G>(liw);            // all lanes are done reading the old knowledge
@@ -511,25 +474,13 @@ __device__ __forceinline__ void rollout_group_body(const EngineParams &P, int T,
         }
         if constexpr (!CALLER_ACTIONS) {
             if (lane == 0) {
-                if (done) done[(long long)t * N + env] = bits ? 1 : 0;
-                if (actions_out) actions_out[(long long)t * N + env] = (uint8_t)action;
+                if (ro.done) ro.done[(long long)t * N + env] = bits ? 1 : 0;
+                if (ro.actions_out) ro.actions_out[(long long)t * N + env] = (uint8_t)action;
             }
         }
         group_sync<G>(liw);   // lane 0's counter store and every lane's S stores are visible to the next step
     }
     if (lane == 0) P.states[env] = st;
-}
-template <int G, int MINB>
-__global__ void __launch_bounds__(kBlock, MINB) rollout_kernel(const __grid_constant__ EngineParams P, int T, uint32_t t0,
-                                                            float *obs, float *obs_last, float *reward, uint8_t *done,
-                                                            uint8_t *actions_out, float *reward_scratch,
-                                                            uint8_t *term_scratch, uint8_t *trunc_scratch) {
-    rollout_group_body<G, false>(P, T, t0, obs, obs_last, reward, done, actions_out, reward_scratch, nullptr);
-}
-template <int G, int MINB>
-__global__ void __launch_bounds__(kBlock, MINB) rollout_actions_kernel(const __grid_constant__ EngineParams P, int T,
-                                                                    const __grid_constant__ RolloutIO ro) {
-    rollout_group_body<G, true>(P, T, 0u, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, &ro);
 }
 
 template <int G>
@@ -608,8 +559,8 @@ __global__ void __launch_bounds__(kBlock, 6) simple_step_tpe_kernel(const __grid
     }
 }
 
-template <int G, int MINB>
-__global__ void __launch_bounds__(kBlock, MINB) simple_step_kernel(EngineParams P, StepIO io) {
+template <int G>
+__global__ void __launch_bounds__(kBlock, 8) simple_step_kernel(EngineParams P, StepIO io) {
     asm volatile("griddepcontrol.launch_dependents;");
     const long long gid = (long long)blockIdx.x * kBlock + threadIdx.x;
     asm volatile("griddepcontrol.wait;" ::: "memory");      // programmatic dependent launch, as in step_call_kernel
@@ -721,14 +672,10 @@ struct nav3d_engine {
     float *d_reward = nullptr, *d_obs = nullptr;
     uint8_t *d_term = nullptr, *d_trunc = nullptr;
     long long *d_actions = nullptr;
-    int minb = 0;               // __launch_bounds__ min CTAs/SM variant of the step kernel (tuning knob)
     bool simple = false;        // NAV3D_ENV_SIMPLE
     int simple_stride = 0;      // simpleEnv, lanes_per_env == 1: floats per staged row (odd: conflict-free), 0 = not staged
-    bool tpe_staged = true;     // thread-per-env kernels: rows staged in shared memory, marking by the warp (NAV3D_TPE_STAGED)
-    int tpe_block = 64;         // their CTA size (NAV3D_TPE_BLOCK)
     bool reset_seen = false;    // a nav3d_reset (or nav3d_restore / nav3d_load_envs) call has been made since the rooms were loaded
     unsigned long long signature = 0;   // engine signature of env-state blobs (nav3d_core.cuh sig_engine / sig_room)
-    bool pdl = true;            // programmatic dependent launch of the step kernel (NAV3D_PDL=0 switches it off)
     float *d_dist_lut = nullptr;
     cudaStream_t own_stream = nullptr;
     static constexpr int kHostChunks = 4;          // nav3d_step_host pipeline depth
@@ -780,6 +727,16 @@ unsigned grid_for(long long n_groups, int G) {
     return (unsigned)((threads + kBlock - 1) / kBlock);
 }
 
+// Launch shape of the thread-per-env step and rollout kernels over n envs: one marking list per warp in dynamic shared memory.
+struct TpeLaunch {
+    unsigned grid, block;
+    size_t smem;
+};
+TpeLaunch tpe_launch(const EngineParams &P, long long n) {
+    return {(unsigned)((n + kTpeBlock - 1) / kTpeBlock), (unsigned)kTpeBlock,
+            (size_t)(kTpeBlock / 32) * P.mark_cap * sizeof(uint32_t)};
+}
+
 int check_ready(const nav3d_engine *e) {
     if (!e) return fail(NAV3D_ERR_INVALID, "engine is NULL");
     if (e->h_rooms.empty()) return fail(NAV3D_ERR_INVALID, "no rooms loaded: call nav3d_load_rooms first");
@@ -824,11 +781,6 @@ int nav3d_create(const nav3d_config *cfg, nav3d_engine **out) {
     if (!e) return fail(NAV3D_ERR_NOMEM, "out of host memory");
     e->cfg = *cfg;
     e->G = G;
-    e->minb = (cfg->env_kind == NAV3D_ENV_SIMPLE || G > 1) ? 8 : 3;
-    if (const char *mb = getenv("NAV3D_MINB")) { if (atoi(mb) > 0) e->minb = atoi(mb); }   // tuning knob (tools/*sweep.sh)
-    if (const char *pd = getenv("NAV3D_PDL")) e->pdl = atoi(pd) != 0;
-    if (const char *v = getenv("NAV3D_TPE_STAGED")) e->tpe_staged = atoi(v) != 0;
-    if (const char *v = getenv("NAV3D_TPE_BLOCK")) e->tpe_block = atoi(v) == 128 ? 128 : 64;
     const size_t N = (size_t)cfg->n_envs;
     cudaError_t err = cudaSuccess;
     if ((err = cudaMalloc(&e->d_states, N * sizeof(EnvState))) != cudaSuccess ||
@@ -850,9 +802,8 @@ int nav3d_create(const nav3d_config *cfg, nav3d_engine **out) {
     e->simple = cfg->env_kind == NAV3D_ENV_SIMPLE;
     if (e->simple && G == 1 && simple_dim <= 95) {
         e->simple_stride = simple_dim;          // 6L+7 is odd: 32 rows at this stride fall into 32 different banks
-        if (!e->tpe_staged) e->simple_stride = 0;
-        else cudaFuncSetAttribute(simple_step_tpe_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                  (int)(kBlock * e->simple_stride * sizeof(float)));
+        cudaFuncSetAttribute(simple_step_tpe_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                             (int)(kBlock * e->simple_stride * sizeof(float)));
     }
     P.obs_dim = e->simple ? 6 * cfg->local_map_length + 7 : kObsDim;
     if (e->simple) {
@@ -941,15 +892,14 @@ int nav3d_load_rooms(nav3d_engine *e, int32_t n_rooms, const nav3d_room_desc *ro
     if (!e->simple && max_k / 4 > 65536)          // a marking task names its tile by a 16-bit word index (MarkQueue)
         return fail(NAV3D_ERR_UNSUPPORTED, "room too large for the marking-task encoding (K volume above 65 536 words)");
     if (!e->simple) {
-        // The default thread-per-env kernels: ask for no more shared memory than their 8 CTAs per SM need, so that the rest
-        // of the 256 KB stays L1 (experiment knob NAV3D_CARVEOUT = percent of the maximum shared memory; 0 = driver's choice)
-        const size_t per_cta = 7680 + 2 * e->P.mark_cap * sizeof(uint32_t) + 1024;
-        int pct = (int)((8 * per_cta * 100 + 228 * 1024 - 1) / (228 * 1024));
-        if (const char *v = getenv("NAV3D_CARVEOUT")) pct = atoi(v);
-        if (pct > 0 && pct <= 100) {
-            cudaFuncSetAttribute(step_tpe_kernel<64, 8, true>, cudaFuncAttributePreferredSharedMemoryCarveout, pct);
-            cudaFuncSetAttribute(rollout_tpe_kernel<64, 8, true>, cudaFuncAttributePreferredSharedMemoryCarveout, pct);
-            cudaFuncSetAttribute(rollout_actions_tpe_kernel<64, 8>, cudaFuncAttributePreferredSharedMemoryCarveout, pct);
+        // The thread-per-env step and rollout kernels: ask for no more shared memory than their 8 CTAs per SM need, so that
+        // the rest of the 256 KB stays L1 (carve-out = percent of the maximum shared memory)
+        const size_t per_cta = 7680 + tpe_launch(e->P, e->cfg.n_envs).smem + 1024;
+        const int pct = (int)((kTpeMinBlocks * per_cta * 100 + 228 * 1024 - 1) / (228 * 1024));
+        if (pct <= 100) {
+            cudaFuncSetAttribute(step_tpe_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, pct);
+            cudaFuncSetAttribute(rollout_tpe_kernel<false>, cudaFuncAttributePreferredSharedMemoryCarveout, pct);
+            cudaFuncSetAttribute(rollout_tpe_kernel<true>, cudaFuncAttributePreferredSharedMemoryCarveout, pct);
         }
     }
     size_t ovf_off = align_up(max_k, 128), stride = ovf_off + align_up(max_cells, 128);
@@ -1080,12 +1030,11 @@ int nav3d_reset(nav3d_engine *e, const int32_t *env_ids, int32_t n, const int32_
     NvtxRange range("nav3d_reset");
     e->reset_seen = true;
     cudaStream_t s = (cudaStream_t)stream;
-    int rc = NAV3D_OK;
-    if (!e->simple && e->G == 1)
-        reset_tpe_kernel<<<grid_for(n, 1), kBlock, (kBlock / 32) * e->P.mark_cap * sizeof(uint32_t), s>>>(e->P, env_ids, n, picks, obs);
-    else rc = dispatch_lanes(e->G, [&](auto g) {
+    const int rc = dispatch_lanes(e->G, [&](auto g) {
         constexpr int G = decltype(g)::value;
         if (e->simple) simple_reset_kernel<G><<<grid_for(n, G), kBlock, 0, s>>>(e->P, env_ids, n, picks, obs);
+        else if constexpr (G == 1)
+            reset_tpe_kernel<<<grid_for(n, 1), kBlock, (kBlock / 32) * e->P.mark_cap * sizeof(uint32_t), s>>>(e->P, env_ids, n, picks, obs);
         else reset_kernel<G><<<grid_for(n, G), kBlock, 0, s>>>(e->P, env_ids, n, picks, obs);
         return NAV3D_OK;
     });
@@ -1102,51 +1051,51 @@ namespace {
 // Launch the step of envs [env0, env0 + n) on `s` (the whole engine: env0 = 0, n = n_envs).
 int launch_step(nav3d_engine *e, StepIO io, int env0, int n, cudaStream_t s) {
     io.env0 = env0; io.env_n = n;
-    const int minb = e->minb;
     int rc = dispatch_lanes(e->G, [&](auto g) {
         constexpr int G = decltype(g)::value;
-        const unsigned grid = grid_for(n, G);
         cudaLaunchConfig_t cfg{};
-        cfg.gridDim = dim3(grid); cfg.blockDim = dim3(kBlock); cfg.dynamicSmemBytes = 0; cfg.stream = s;
+        cfg.gridDim = dim3(grid_for(n, G)); cfg.blockDim = dim3(kBlock); cfg.dynamicSmemBytes = 0; cfg.stream = s;
         cudaLaunchAttribute attr[1];
         attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-        attr[0].val.programmaticStreamSerializationAllowed = e->pdl ? 1 : 0;
+        attr[0].val.programmaticStreamSerializationAllowed = 1;
         cfg.attrs = attr; cfg.numAttrs = 1;
         if (e->simple) {
             if (G == 1 && e->simple_stride > 0) {      // thread per env, staged rows (6L+7 <= 95 floats)
                 cfg.dynamicSmemBytes = (size_t)kBlock * e->simple_stride * sizeof(float);
                 cudaLaunchKernelEx(&cfg, simple_step_tpe_kernel, e->P, io, e->simple_stride);
-                return NAV3D_OK;
+            } else {
+                cudaLaunchKernelEx(&cfg, simple_step_kernel<G>, e->P, io);
             }
-            if (minb == 6) cudaLaunchKernelEx(&cfg, simple_step_kernel<G, 6>, e->P, io);
-            else cudaLaunchKernelEx(&cfg, simple_step_kernel<G, 8>, e->P, io);
-            return NAV3D_OK;
+        } else if constexpr (G == 1) {                 // thread per env: staged, coalesced observation stores
+            const TpeLaunch l = tpe_launch(e->P, n);
+            cfg.gridDim = dim3(l.grid); cfg.blockDim = dim3(l.block); cfg.dynamicSmemBytes = l.smem;
+            cudaLaunchKernelEx(&cfg, step_tpe_kernel, e->P, io);
+        } else {
+            cudaLaunchKernelEx(&cfg, step_call_kernel<G>, e->P, io);
         }
-        if (G == 1) {                                  // thread per env: staged, coalesced observation stores
-            const bool staged = e->tpe_staged;
-            // Default: 64-thread CTAs, 8 per SM (128 registers, 16 warps per SM) — the sweep of DESIGN.md §6; NAV3D_TPE_BLOCK=128
-            // selects the 128-thread kernels (NAV3D_MINB 3: 168 registers / 12 warps, 4: 128 / 16)
-            const int tblock = e->tpe_block;
-            cfg.dynamicSmemBytes = (size_t)(tblock / 32) * e->P.mark_cap * sizeof(uint32_t);   // one marking list per warp
-            if (tblock == 64 && staged) {
-                cfg.gridDim = dim3((unsigned)((n + 63) / 64)); cfg.blockDim = dim3(64);
-                cudaLaunchKernelEx(&cfg, step_tpe_kernel<64, 8, true>, e->P, io);
-                return NAV3D_OK;
-            }
-            switch (minb * 2 + (staged ? 1 : 0)) {
-                case 8: cudaLaunchKernelEx(&cfg, step_tpe_kernel<128, 4, false>, e->P, io); break;
-                case 9: cudaLaunchKernelEx(&cfg, step_tpe_kernel<128, 4, true>, e->P, io); break;
-                case 6: cudaLaunchKernelEx(&cfg, step_tpe_kernel<128, 3, false>, e->P, io); break;
-                default: cudaLaunchKernelEx(&cfg, step_tpe_kernel<128, 3, true>, e->P, io); break;
-            }
-            return NAV3D_OK;
-        }
-        if (minb == 6) cudaLaunchKernelEx(&cfg, step_call_kernel<G, 6>, e->P, io);
-        else cudaLaunchKernelEx(&cfg, step_call_kernel<G, 8>, e->P, io);
         return NAV3D_OK;
     });
     if (rc) return rc;
     e->launches += 1;
+    CUDA_TRY(cudaGetLastError());
+    return NAV3D_OK;
+}
+
+// Launch the fused T-step rollout of all envs (CubicEnv) on `s`: caller-supplied or Philox actions.
+template <bool CALLER_ACTIONS>
+int launch_rollout(nav3d_engine *e, int T, const RolloutIO &ro, cudaStream_t s) {
+    int rc = dispatch_lanes(e->G, [&](auto g) {
+        constexpr int G = decltype(g)::value;
+        if constexpr (G == 1) {
+            const TpeLaunch l = tpe_launch(e->P, e->cfg.n_envs);
+            rollout_tpe_kernel<CALLER_ACTIONS><<<l.grid, l.block, l.smem, s>>>(e->P, T, ro);
+        } else {
+            rollout_kernel<G, CALLER_ACTIONS><<<grid_for(e->cfg.n_envs, G), kBlock, 0, s>>>(e->P, T, ro);
+        }
+        return NAV3D_OK;
+    });
+    if (rc) return rc;
+    e->launches++;
     CUDA_TRY(cudaGetLastError());
     return NAV3D_OK;
 }
@@ -1221,30 +1170,9 @@ int nav3d_rollout_random(nav3d_engine *e, int32_t T, uint32_t t0, float *obs, fl
         return fail(NAV3D_ERR_INVALID, "obs must be 16-byte aligned");
     NAV3D_DEVICE(e);
     NvtxRange range("nav3d_rollout_random");
-    cudaStream_t s = (cudaStream_t)stream;
-    int rc = dispatch_lanes(e->G, [&](auto g) {
-        constexpr int G = decltype(g)::value;
-        if (G == 1) {
-            const int tblock = e->tpe_block;
-            if (tblock == 64)
-                rollout_tpe_kernel<64, 8, true><<<(unsigned)((e->cfg.n_envs + 63) / 64), 64, 2 * e->P.mark_cap * sizeof(uint32_t), s>>>(e->P, T, t0, obs, obs_last,
-                                                                                                  reward, done, actions_out);
-            else if (e->minb == 4)
-                rollout_tpe_kernel<128, 4, true><<<grid_for(e->cfg.n_envs, 1), kBlock, 4 * e->P.mark_cap * sizeof(uint32_t), s>>>(e->P, T, t0, obs, obs_last, reward,
-                                                                                            done, actions_out);
-            else
-                rollout_tpe_kernel<128, 3, true><<<grid_for(e->cfg.n_envs, 1), kBlock, 4 * e->P.mark_cap * sizeof(uint32_t), s>>>(e->P, T, t0, obs, obs_last, reward,
-                                                                                            done, actions_out);
-            return NAV3D_OK;
-        }
-        rollout_kernel<G, 6><<<grid_for(e->cfg.n_envs, G), kBlock, 0, s>>>(e->P, T, t0, obs, obs_last, reward, done, actions_out,
-                                                                           e->d_reward, e->d_term, e->d_trunc);
-        return NAV3D_OK;
-    });
-    if (rc) return rc;
-    e->launches++;
-    CUDA_TRY(cudaGetLastError());
-    return NAV3D_OK;
+    RolloutIO ro{};
+    ro.obs = obs; ro.obs_last = obs_last; ro.reward = reward; ro.done = done; ro.actions_out = actions_out; ro.t0 = t0;
+    return launch_rollout<false>(e, T, ro, (cudaStream_t)stream);
 }
 
 int nav3d_rollout_actions(nav3d_engine *e, int32_t T, const uint8_t *actions, float *obs, float *obs_last, float *reward,
@@ -1260,27 +1188,10 @@ int nav3d_rollout_actions(nav3d_engine *e, int32_t T, const uint8_t *actions, fl
     if (T == 0) return NAV3D_OK;
     NAV3D_DEVICE(e);
     NvtxRange range("nav3d_rollout_actions");
-    RolloutIO ro;
+    RolloutIO ro{};
     ro.actions = actions; ro.obs = obs; ro.obs_last = obs_last; ro.reward = reward; ro.reward64 = reward64;
     ro.terminated = terminated; ro.truncated = truncated; ro.terminal_obs = terminal_obs; ro.episodes = episodes;
-    cudaStream_t s = (cudaStream_t)stream;
-    const int n = e->cfg.n_envs;
-    int rc = dispatch_lanes(e->G, [&](auto g) {
-        constexpr int G = decltype(g)::value;
-        if constexpr (G == 1) {           // the launch configurations of nav3d_rollout_random
-            const size_t smem = (size_t)(e->tpe_block / 32) * e->P.mark_cap * sizeof(uint32_t);
-            if (e->tpe_block == 64) rollout_actions_tpe_kernel<64, 8><<<(unsigned)((n + 63) / 64), 64, smem, s>>>(e->P, T, ro);
-            else if (e->minb == 4) rollout_actions_tpe_kernel<128, 4><<<grid_for(n, 1), kBlock, smem, s>>>(e->P, T, ro);
-            else rollout_actions_tpe_kernel<128, 3><<<grid_for(n, 1), kBlock, smem, s>>>(e->P, T, ro);
-        } else {
-            rollout_actions_kernel<G, 6><<<grid_for(n, G), kBlock, 0, s>>>(e->P, T, ro);
-        }
-        return NAV3D_OK;
-    });
-    if (rc) return rc;
-    e->launches++;
-    CUDA_TRY(cudaGetLastError());
-    return NAV3D_OK;
+    return launch_rollout<true>(e, T, ro, (cudaStream_t)stream);
 }
 
 int nav3d_get_state(nav3d_engine *e, int32_t *state, void *stream) {

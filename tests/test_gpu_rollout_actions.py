@@ -149,13 +149,6 @@ def test_equals_steps_without_auto_reset(lanes):
     assert ends.max() > 1                    # envs keep stepping past done
 
 
-@pytest.mark.parametrize("minb", [3, 4])
-def test_equals_steps_128_thread_variants(monkeypatch, minb):
-    monkeypatch.setenv("NAV3D_TPE_BLOCK", "128")
-    monkeypatch.setenv("NAV3D_MINB", str(minb))
-    check_equivalence(short_episode_rooms(), n=1013, T=200, seed=minb, lanes=1, pre_steps=0)
-
-
 @pytest.mark.parametrize("outputs", [("reward",), ("flags", "eps"), ("reward64", "tobs"), ("obs",), ("obs", "eps")])
 @pytest.mark.parametrize("lanes", [0, 4])
 def test_obs_last_and_null_outputs(outputs, lanes):

@@ -18,7 +18,7 @@ ncu --set full --clock-control none --import-source on -k regex:rollout -s 19 -c
 # the reports stay on the box (gpurun brings back at most 64 MiB): summaries, raw metric tables and per-line instruction /
 # stall-sample tables are made here
 for r in step_${TAG}_cold step_${TAG}_steady rollout_${TAG}_cold rollout_${TAG}_steady; do
-  case $r in step_*) N=1048576; K=step_tpe_kernelILi64ELi8ELb1E;; *) N=33554432; K=rollout_tpe_kernelILi64ELi8ELb1E;; esac
+  case $r in step_*) N=1048576; K=15step_tpe_kernelE;; *) N=33554432; K=rollout_tpe_kernelILb0E;; esac
   python tools/ncu_summary.py $O/prof_$r.ncu-rep $N > $O/${r}_summary.txt 2>&1
   ncu -i $O/prof_$r.ncu-rep --page raw --csv > $O/${r}_details.csv 2>/dev/null
   python tools/sass_lines.py $O/prof_$r.ncu-rep $K $N 60 > $O/${r}_lines.txt 2>&1

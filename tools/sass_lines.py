@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Warp-instructions executed per SOURCE LINE of one kernel: joins the per-SASS-instruction counts of an .ncu-rep
 (`ncu --set full --import-source on`, read here without a GPU) with the line table of the built library (nvdisasm -g).
-usage: tools/sass_lines.py file.ncu-rep <kernel-substring of the mangled name, e.g. step_call_kernelILi4ELi8> [n_envs] [top]"""
+usage: tools/sass_lines.py file.ncu-rep <kernel-substring of the mangled name, e.g. step_call_kernelILi4E> [n_envs] [top]"""
 import csv, re, subprocess, sys, tempfile, os
 from collections import defaultdict
 from pathlib import Path
