@@ -19,8 +19,9 @@ namespace {
 
 constexpr uint32_t kStreamPolicy = 0x504f4c49u;   // "POLI": counter = (global_env_id, step index, 0, tag)
 
-// One thread per env.  Inverse-CDF sampling on softmax(logits) with u = Philox word / 2^32; the same pass gives
-// log pi(a|s) and the entropy, so the rollout needs no second softmax.
+// One thread per env.  Inverse-CDF sampling on softmax(logits) with u = (Philox word >> 8) / 2^24; the same pass gives
+// log pi(a|s) and the entropy, so the rollout needs no second softmax.  A row may mask actions with -inf as long as one
+// entry is finite: masked actions get weight 0, are never drawn and add 0 to the entropy.
 template <bool GREEDY>
 __global__ void __launch_bounds__(256) sample_actions_kernel(const float *__restrict__ logits, int N, int A,
                                                              uint32_t env_id0, uint32_t step,
@@ -45,7 +46,11 @@ __global__ void __launch_bounds__(256) sample_actions_kernel(const float *__rest
         // step_offset lives in device memory so that a CUDA graph of a whole rollout can be replayed with fresh draws
         const uint32_t idx = step + (step_offset ? *step_offset : 0u);
         philox4x32_10(env_id0 + (uint32_t)n, idx, 0u, kStreamPolicy, seed_lo, seed_hi, u0, u1);
-        const float target = (float)u0 * (1.0f / 4294967296.0f) * sum;       // u in [0, 1)
+        // u = top 24 bits / 2^24 is exact in fp32 and at most 1 - 2^-24, so target < sum, which is the final acc: the walk
+        // always stops inside the loop, on a term with nonzero weight.  ((float)u0 / 2^32 rounds to 1.0 for the top 128
+        // words, and the walk then fell through to A - 1 whatever its weight.)
+        const float u = (float)(u0 >> 8) * 0x1p-24f;
+        const float target = u * sum;
         float acc = 0.f;
         a = A - 1;
         for (int k = 0; k < A; k++) {
@@ -59,7 +64,8 @@ __global__ void __launch_bounds__(256) sample_actions_kernel(const float *__rest
         float h = 0.f;
         for (int k = 0; k < A; k++) {
             const float lp = row[k] - mx - lse;
-            h -= expf(lp) * lp;
+            const float p = expf(lp);
+            if (p > 0.f) h -= p * lp;                // p = 0 (a -inf logit) adds 0, not 0 * -inf = NaN
         }
         entropy[n] = h;
     }

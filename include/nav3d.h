@@ -271,10 +271,13 @@ int nav3d_load_envs(nav3d_engine *e, const int32_t *env_ids, int32_t n, const vo
  * reference's third-party stack (sb3-contrib RecurrentPPO driven by train/Grid_Train.py:198-228), the per-step
  * `distribution.get_actions()/log_prob()` and `RecurrentRolloutBuffer.compute_returns_and_advantage`. ---- */
 
-/* Categorical sampling from policy logits f32[n][n_actions] (row-major).  u = word 0 of Philox4x32-10 with
- * counter = (env_id0 + i, step + *step_offset, 0, 0x504f4c49) and the key of `seed`; action = first k with
- * cumsum(softmax)[k] > u.  step_offset: DEVICE u32[1] or NULL (= 0) — a counter in device memory, so that a CUDA graph
- * that captured a whole rollout draws fresh numbers on every replay.
+/* Categorical sampling from policy logits f32[n][n_actions] (row-major).  u = (word0 >> 8) / 2^24, where word0 is word 0
+ * of Philox4x32-10 with counter = (env_id0 + i, step + *step_offset, 0, 0x504f4c49) (both sums mod 2^32) and the key of
+ * `seed`, so u lies in [0, 1 - 2^-24]; action = first k with cumsum(softmax)[k] > u.  step_offset: DEVICE u32[1] or
+ * NULL (= 0) — a counter in device memory, so that a CUDA graph that captured a whole rollout draws fresh numbers on
+ * every replay.
+ * A logits row may hold -inf entries (masked actions) if at least one entry is finite: masked actions are never drawn
+ * and add 0 to the entropy.  A row containing +inf or NaN gives undefined output.
  * greedy != 0: argmax instead (SB3's deterministic=True, train/evaluate_grid.py:186-191).
  *   actions : int64[n] (directly usable by nav3d_step)   log_prob : f32[n] or NULL   entropy : f32[n] or NULL */
 int nav3d_sample_actions(const float *logits, int32_t n, int32_t n_actions, uint64_t seed, uint32_t env_id0,
