@@ -32,6 +32,9 @@
 //     the neighbour codes.
 #pragma once
 #include <stdint.h>
+#include <algorithm>
+#include <cstdio>
+#include <cstdlib>
 #include <cuda_runtime.h>
 
 #define NAV3D_HD __host__ __device__ __forceinline__
@@ -79,28 +82,71 @@ struct alignas(32) EnvState {      // one 32-byte sector per env: read once, wri
 };
 static_assert(sizeof(EnvState) == 32, "EnvState must be one 32-byte sector");
 
-// Reward constants of compute_reward (CubicEnv.py:169-224); include/nav3d.h nav3d_reward_params mirrors this.  `centi`
-// holds every term except the crash penalty in 1/100 units for the integer episode-return accumulator.
+// Reward constants of compute_reward (CubicEnv.py:169-224); include/nav3d.h nav3d_reward_params mirrors this.  The c_*
+// fields hold the fixed terms except the crash penalty in 1/100 units for the integer episode-return accumulator; the
+// revisit term's cents are rounded from the f64 penalty of each step (step_commit).
 struct RewardParams {
     double step_cost, revisit_unit, revisit_cap, crash_penalty, near_wall_bonus, repeat_bonus, reverse_penalty,
         explore_bonus, finish_bonus, truncation_penalty;
-    int32_t c_step, c_revisit_unit, c_revisit_cap, c_near_wall, c_repeat, c_reverse, c_explore, c_finish, c_trunc;
+    int32_t c_step, c_near_wall, c_repeat, c_reverse, c_explore, c_finish, c_trunc;
 };
 
-// centi-units of one reward term for the integer episode-return accumulator (exact for the reference's constants)
-inline int32_t reward_centi(double v) { return (int32_t)(v * 100.0 + (v < 0 ? -0.5 : 0.5)); }
-// The reference's literals (CubicEnv.py:175, :179-180, :187, :193, :199, :203, :209, :215, :221).
-inline RewardParams reference_reward_params(double crash_penalty) {
+// centi-units of one reward term, rounded half away from zero (exact for multiples of 0.01 up to |v| <= 1e6)
+NAV3D_HD int32_t reward_centi(double v) {
+#ifdef __CUDA_ARCH__
+    const double s = __dmul_rn(v, 100.0);      // not fused with the add below: the host rounds v * 100 first, too
+#else
+    const double s = v * 100.0;
+#endif
+    return (int32_t)(s + (v < 0 ? -0.5 : 0.5));
+}
+
+// v = the ten fields of nav3d_reward_params in declaration order
+inline RewardParams reward_params_from(const double v[10]) {
     RewardParams w;
-    w.step_cost = -0.05; w.revisit_unit = 0.02; w.revisit_cap = 0.5; w.crash_penalty = crash_penalty;
-    w.near_wall_bonus = 0.15; w.repeat_bonus = 0.05; w.reverse_penalty = 0.5; w.explore_bonus = 1.0;
-    w.finish_bonus = 100.0; w.truncation_penalty = -5.0;
-    w.c_step = reward_centi(w.step_cost); w.c_revisit_unit = reward_centi(w.revisit_unit);
-    w.c_revisit_cap = reward_centi(w.revisit_cap); w.c_near_wall = reward_centi(w.near_wall_bonus);
+    w.step_cost = v[0]; w.revisit_unit = v[1]; w.revisit_cap = v[2]; w.crash_penalty = v[3]; w.near_wall_bonus = v[4];
+    w.repeat_bonus = v[5]; w.reverse_penalty = v[6]; w.explore_bonus = v[7]; w.finish_bonus = v[8];
+    w.truncation_penalty = v[9];
+    w.c_step = reward_centi(w.step_cost); w.c_near_wall = reward_centi(w.near_wall_bonus);
     w.c_repeat = reward_centi(w.repeat_bonus); w.c_reverse = reward_centi(w.reverse_penalty);
     w.c_explore = reward_centi(w.explore_bonus); w.c_finish = reward_centi(w.finish_bonus);
     w.c_trunc = reward_centi(w.truncation_penalty);
     return w;
+}
+// The reference's literals (CubicEnv.py:175, :179-180, :187, :193, :199, :203, :209, :215, :221).
+inline RewardParams reference_reward_params(double crash_penalty) {
+    const double v[10] = {-0.05, 0.02, 0.5, crash_penalty, 0.15, 0.05, 0.5, 1.0, 100.0, -5.0};
+    return reward_params_from(v);
+}
+
+// Why a parameter set of finite values within [-1e6, 1e6] cannot be honoured, or nullptr (include/nav3d.h,
+// nav3d_set_reward_params).
+//  - The record keeps the agent cell's visit count saturated at 255, so min(count * unit, cap) must not change once the
+//    count passes 255: unit == 0, or unit > 0 and 255 * unit >= cap.
+//  - ret_centi is an int32: the largest |cents| one step can add, over 65 535 steps, plus one finish and one truncation
+//    term, must fit.  Both the count (1..255) and the penalty are monotone, so the revisit extremes are at counts 1 and 255.
+inline const char *reward_params_reject(const RewardParams &w) {
+    if (!(w.revisit_unit == 0.0 || (w.revisit_unit > 0.0 && 255.0 * w.revisit_unit >= w.revisit_cap)))
+        return "revisit_unit must be 0, or positive with 255 * revisit_unit >= revisit_cap: visit counts saturate at 255, "
+               "so min(count * revisit_unit, revisit_cap) must not change past count 255";
+    auto a = [](long long c) { return c < 0 ? -c : c; };
+    const double p1 = w.revisit_unit < w.revisit_cap ? w.revisit_unit : w.revisit_cap;
+    const double p255 = 255.0 * w.revisit_unit < w.revisit_cap ? 255.0 * w.revisit_unit : w.revisit_cap;
+    const long long rev = std::max(a(reward_centi(p1)), a(reward_centi(p255)));
+    const long long per_step = a(w.c_step) + rev + a(w.c_near_wall) + std::max(a(w.c_repeat), a(w.c_reverse)) + a(w.c_explore);
+    if (65535LL * per_step + a(w.c_finish) + a(w.c_trunc) > 2147483647LL)
+        return "the largest episode return these parameters allow (65 535 steps) does not fit the int32 accumulator of "
+               "1/100 units";
+    return nullptr;
+}
+
+// Python's round(x, 2): the exact binary value of x rounded to two decimals (ties to even), as glibc's printf does, then
+// parsed back.  rint(x * 100) / 100 is not the same: 0.175 * 100 rounds onto the tie 17.5 and gives 0.18, while
+// round(0.175, 2) is 0.17 (0.175 is slightly below 0.175 in binary).
+inline double py_round2(double x) {
+    char buf[64];
+    std::snprintf(buf, sizeof buf, "%.2f", x);
+    return std::strtod(buf, nullptr);
 }
 
 struct EngineParams {
@@ -179,6 +225,11 @@ template <typename T> NAV3D_HD T ldg(const T *p) {
 #endif
 }
 NAV3D_HD int imin(int a, int b) { return a < b ? a : b; }
+// a + b clamped to the int32 range (the episode-return accumulator of an env stepped on past done, auto_reset = 0)
+NAV3D_HD int add_saturate(int a, int b) {
+    const long long s = (long long)a + b;
+    return s > 2147483647LL ? 2147483647 : (s < -2147483647LL - 1 ? (int)(-2147483647LL - 1) : (int)s);
+}
 NAV3D_HD int imax(int a, int b) { return a > b ? a : b; }
 // Streaming (evict-first) stores for data that is written once and not read again by this engine (observations, rewards,
 // flags): keeps them from evicting the per-env knowledge lines that the NEXT step will touch again from L2.
@@ -766,6 +817,7 @@ struct StepCtx {                   // what the second half needs; identical in e
     EnvState st;                   // the record the step started from
     int x, y, z, facing, a, c_new, down;
     uint32_t flags, step_count, visited, n_free, blocked6;
+    uint32_t ovf_at;               // G > 1: offset in the env's block of the agent cell's overflow byte
     bool bumped, explored, done, truncated, will_reset, near_wall;
 };
 
@@ -822,8 +874,11 @@ NAV3D_HD uint32_t step_lane(const EngineParams &P, const StepIO &io, int env, in
 
     const Rays r = cast_rays(P, R, x, y, z);
     c.down = r.down; c.blocked6 = r.blocked6; c.near_wall = r.near_wall != 0;
-    if (c.c_new >= kOverflowBase && lane == 0 && !c.will_reset)
-        envk[P.ovf_off + ovf_index(R, x, y, z)] = (uint8_t)(c.c_new - kOverflowBase);
+    // The agent cell's exact count past 28.  With G > 1 the sibling lanes read the byte of the cell they move into
+    // above, in the same step, so the store waits for step_commit, after the group's reduction.
+    if (G == 1) {
+        if (c.c_new >= kOverflowBase && !c.will_reset) envk[P.ovf_off + ovf_index(R, x, y, z)] = (uint8_t)(c.c_new - kOverflowBase);
+    } else c.ovf_at = P.ovf_off + ovf_index(R, x, y, z);
 
     // get_obs (:122)
     float *orow = io.obs ? io.obs + row * kObsDim : nullptr;
@@ -849,8 +904,9 @@ NAV3D_HD void step_commit(const EngineParams &P, const StepIO &io, int env, int 
     // compute_reward (:169-224), same operations in the same order, f64
     double rew = w.step_cost;
     const double pen = (double)c.c_new * w.revisit_unit;
-    rew -= (pen < w.revisit_cap) ? pen : w.revisit_cap;
-    int cents = w.c_step - imin(w.c_revisit_unit * c.c_new, w.c_revisit_cap);
+    const double revisit = (pen < w.revisit_cap) ? pen : w.revisit_cap;
+    rew -= revisit;
+    int cents = w.c_step - reward_centi(revisit);
     uint32_t bump_count = st.bump_count;
     if (c.bumped) {
         flags |= kLastBump;
@@ -865,8 +921,10 @@ NAV3D_HD void step_commit(const EngineParams &P, const StepIO &io, int env, int 
     if (c.explored) { rew += w.explore_bonus; cents += w.c_explore; }
     if (c.done) { flags |= kDone; rew += w.finish_bonus; cents += w.c_finish; }
     if (c.truncated) { rew += w.truncation_penalty; cents += w.c_trunc; }
-    const int ret_centi = st.ret_centi + cents;
+    const int ret_centi = add_saturate(st.ret_centi, cents);
 
+    if (G > 1 && writer && c.c_new >= kOverflowBase && !c.will_reset)
+        P.know[(unsigned long long)env * P.env_stride + c.ovf_at] = (uint8_t)(c.c_new - kOverflowBase);
     if (writer) {
         if (!REG_STATE || io.reward) store_stream(io.reward + row, (float)rew);
         if (io.reward64) io.reward64[row] = rew;

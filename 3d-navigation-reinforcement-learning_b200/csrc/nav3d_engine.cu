@@ -810,7 +810,7 @@ int nav3d_create(const nav3d_config *cfg, nav3d_engine **out) {
         // distances of simpleEnv: round(count * cell_size, 2) (simpleEnv.py:337) then float32
         std::vector<float> lut((size_t)cfg->local_map_length + 1);
         for (int c = 0; c <= cfg->local_map_length; c++)
-            lut[(size_t)c] = (float)(std::nearbyint((double)c * cfg->cell_size * 100.0) / 100.0);
+            lut[(size_t)c] = (float)py_round2((double)c * cfg->cell_size);
         if ((err = cudaMalloc(&e->d_dist_lut, lut.size() * sizeof(float))) != cudaSuccess ||
             (err = cudaMemcpy(e->d_dist_lut, lut.data(), lut.size() * sizeof(float), cudaMemcpyHostToDevice)) != cudaSuccess) {
             nav3d_destroy(e);
@@ -980,15 +980,8 @@ int nav3d_set_reward_params(nav3d_engine *e, const nav3d_reward_params *p) {
     const double v[10] = {p->step_cost, p->revisit_unit, p->revisit_cap, p->crash_penalty, p->near_wall_bonus, p->repeat_bonus,
                           p->reverse_penalty, p->explore_bonus, p->finish_bonus, p->truncation_penalty};
     for (double x : v) if (!std::isfinite(x) || std::fabs(x) > 1e6) return fail(NAV3D_ERR_INVALID, "reward parameter out of range");
-    RewardParams w = reference_reward_params(p->crash_penalty);
-    w.step_cost = p->step_cost; w.revisit_unit = p->revisit_unit; w.revisit_cap = p->revisit_cap;
-    w.near_wall_bonus = p->near_wall_bonus; w.repeat_bonus = p->repeat_bonus; w.reverse_penalty = p->reverse_penalty;
-    w.explore_bonus = p->explore_bonus; w.finish_bonus = p->finish_bonus; w.truncation_penalty = p->truncation_penalty;
-    w.c_step = reward_centi(w.step_cost); w.c_revisit_unit = reward_centi(w.revisit_unit);
-    w.c_revisit_cap = reward_centi(w.revisit_cap); w.c_near_wall = reward_centi(w.near_wall_bonus);
-    w.c_repeat = reward_centi(w.repeat_bonus); w.c_reverse = reward_centi(w.reverse_penalty);
-    w.c_explore = reward_centi(w.explore_bonus); w.c_finish = reward_centi(w.finish_bonus);
-    w.c_trunc = reward_centi(w.truncation_penalty);
+    const RewardParams w = reward_params_from(v);
+    if (const char *why = reward_params_reject(w)) return fail(NAV3D_ERR_UNSUPPORTED, std::string("nav3d_set_reward_params: ") + why);
     e->P.rw = w;
     return NAV3D_OK;
 }

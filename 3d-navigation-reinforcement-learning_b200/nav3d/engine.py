@@ -47,6 +47,11 @@ class Engine:
         self.n_envs = int(n_envs)
         self.local_map_length = int(local_map_length)
         self.crash_penalty = float(crash_penalty)
+        p = _lib.RewardParams()
+        self._lib.nav3d_reward_params_default(C.byref(p))
+        p.crash_penalty = self.crash_penalty
+        # the values the engine's kernels use (nav3d_reward_params fields), kept in step with set_reward_params
+        self.reward_params = {f: float(getattr(p, f)) for f, _ in _lib.RewardParams._fields_}
         self.auto_reset = bool(auto_reset)
         self.seed = int(seed)
         self.env_id0 = int(env_id0)
@@ -84,16 +89,16 @@ class Engine:
 
     def set_reward_params(self, **kwargs):
         """Override literals of ``compute_reward`` (reference ``envs/CubicEnv.py:169-224``); names are the fields of
-        ``nav3d_reward_params``.  Unnamed ones keep their current reference default."""
-        p = _lib.RewardParams()
-        self._lib.nav3d_reward_params_default(C.byref(p))
-        p.crash_penalty = self.crash_penalty
+        ``nav3d_reward_params``.  Unnamed ones keep the engine's current values (``reward_params``).  A set the engine
+        cannot honour raises ``Nav3dError`` and leaves the current values in place."""
+        p = _lib.RewardParams(**self.reward_params)
         for k, v in kwargs.items():
             if not hasattr(p, k):
                 raise TypeError(f"unknown reward parameter {k!r}")
             setattr(p, k, float(v))
         check(self._lib.nav3d_set_reward_params(self._h, C.byref(p)))
-        self.crash_penalty = float(p.crash_penalty)
+        self.reward_params = {f: float(getattr(p, f)) for f, _ in _lib.RewardParams._fields_}
+        self.crash_penalty = self.reward_params["crash_penalty"]
 
     def free_cell(self, room: int, k: int):
         xyz = (C.c_int32 * 3)()

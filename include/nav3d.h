@@ -96,8 +96,27 @@ typedef struct {
  *            + (bumped ? crash_penalty : [was_near_wall] near_wall_bonus + [same horizontal action again] repeat_bonus
  *                                        - [backwards twice] reverse_penalty)
  *            + [first visit] explore_bonus + [>= 84 % explored] finish_bonus + [step limit] truncation_penalty
- * nav3d_episode.episode_return is accumulated in 1/100 units: exact when every constant except crash_penalty is a
- * multiple of 0.01 (true for the reference's), rounded per term otherwise. */
+ *
+ * Episode return.  Each step adds to an int32 in 1/100 units (nav3d_get_state column 15) every term but the crash
+ * penalty, each rounded on its own: round(100 * v) half away from zero, for the revisit term of the f64 value
+ * min(visit_count * revisit_unit, revisit_cap) of that step.  nav3d_episode.episode_return is then
+ * (float)(centi / 100.0 + bump_count * crash_penalty).  It equals the f64 sum of the episode's rewards up to f64 and
+ * f32 rounding when every parameter except crash_penalty is a multiple of 0.01 (true for the reference's); in general
+ *     |episode_return - sum of rewards| <= 0.005 * (5 * length + 2) + 2^-24 * |episode_return| + 1e-3
+ * (at most five rounded terms a step, plus the finish and truncation terms).  The accumulator saturates at the int32
+ * limits instead of wrapping; only an env stepped on past done with auto_reset = 0 can reach them (about 2.3e5 steps
+ * at the defaults), since every accepted parameter set keeps one episode within them.
+ *
+ * nav3d_set_reward_params checks, and fails with NAV3D_ERR_UNSUPPORTED (nav3d_last_error names the rule) for:
+ *   - saturation: the visit count of the agent's cell saturates at 255, so the set must give the same
+ *     min(count * revisit_unit, revisit_cap) for every count past 255: revisit_unit == 0, or revisit_unit > 0 and
+ *     255.0 * revisit_unit >= revisit_cap (in f64);
+ *   - overflow: 65535 * M + |c(finish_bonus)| + |c(truncation_penalty)| must fit an int32, where c(v) is a term in
+ *     1/100 units as above and M, the largest |cents| of one step, is |c(step_cost)| + max(|c(min(revisit_unit,
+ *     revisit_cap))|, |c(min(255 * revisit_unit, revisit_cap))|) + |c(near_wall_bonus)| + max(|c(repeat_bonus)|,
+ *     |c(reverse_penalty)|) + |c(explore_bonus)|.
+ * A value that is not finite or exceeds 1e6 in magnitude gives NAV3D_ERR_INVALID.  A rejected set leaves the engine's
+ * parameters as they were. */
 typedef struct {
     double step_cost;             /* -0.05  :175 */
     double revisit_unit;          /*  0.02  :179 */
@@ -132,7 +151,11 @@ int nav3d_create(const nav3d_config *cfg, nav3d_engine **out);
 void nav3d_destroy(nav3d_engine *e);
 
 void nav3d_reward_params_default(nav3d_reward_params *out);
-/* Takes effect from the next step on; may be called at any time (host-side copy, no device work). */
+/* Takes effect from the next launch on; may be called at any time, mid-episode too (host-side copy, no device work).
+ * The parameters are copied into each kernel's launch arguments, so a CUDA graph captured before this call keeps
+ * replaying with the values it captured: capture the graph again after changing them.  Env-state blobs hold no reward
+ * parameters: a loaded env continues with those of the engine it is loaded into.  CubicEnv only (NAV3D_ERR_UNSUPPORTED
+ * for simpleEnv).  The accepted sets are described at nav3d_reward_params. */
 int nav3d_set_reward_params(nav3d_engine *e, const nav3d_reward_params *params);
 
 /* The room table: replaces the per-reset text parse + free-cell scan of load_room (envs/CubicEnv.py:402-459).
@@ -212,7 +235,7 @@ int nav3d_rollout_actions(nav3d_engine *e, int32_t T, const uint8_t *actions, fl
  * visited_count/bump_count/done evaluate_grid.py:216-218, ...).  DEVICE int32[n_envs][NAV3D_STATE_INTS]:
  *  0 x  1 y  2 z  3 facing  4 visited_count  5 bump_count  6 step_count  7 near_wall  8 was_near_wall  9 last_bump
  * 10 done  11 cells_insight_down  12 last_action  13 room index  14 episode number  15 return so far, in 1/100 units,
- *    excluding crash penalties */
+ *    excluding crash penalties; CubicEnv: saturating at the int32 limits (see nav3d_reward_params) */
 int nav3d_get_state(nav3d_engine *e, int32_t *state, void *stream);
 /* self.internal_grid of one env (CubicEnv.py:84-85) rebuilt from the packed representation, DEVICE int16
  * [width][depth][height] of the env's current room (C order).   Visit counters saturate at 255. */

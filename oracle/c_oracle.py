@@ -49,6 +49,9 @@ def lib():
         "orc_vec_step": (None, [P, P, P, P, P, P, P, P, P, P, P]),
         "orc_vec_rollout_random": (C.c_long, [P, I, C.c_uint32, P, P]),
         "orc_vec_rollout_random_obs": (C.c_long, [P, I, C.c_uint32, P]),
+        "orc_cubic_set_reward": (None, [P, P]), "orc_cubic_ret_centi": (C.c_long, [P]),
+        "orc_cubic_episode_return": (C.c_float, [P]), "orc_py_round2": (D, [D]),
+        "orc_vec_set_reward": (None, [P, P]), "orc_vec_ret_centi": (None, [P, P]), "orc_vec_ep_return32": (None, [P, P]),
         "orc_set_threads": (None, [I]), "orc_get_threads": (I, []), "orc_hw_threads": (I, []),
     }
     for name, (res, args) in sig.items():
@@ -60,6 +63,27 @@ def lib():
 
 def _p(a):
     return None if a is None else C.c_void_p(a.ctypes.data)
+
+
+REWARD_FIELDS = ("step_cost", "revisit_unit", "revisit_cap", "crash_penalty", "near_wall_bonus", "repeat_bonus",
+                 "reverse_penalty", "explore_bonus", "finish_bonus", "truncation_penalty")
+REWARD_DEFAULTS = dict(zip(REWARD_FIELDS, (-0.05, 0.02, 0.5, -2.0, 0.15, 0.05, 0.5, 1.0, 100.0, -5.0)))
+
+
+def reward_values(reward=None, crash_penalty: float = -2.0) -> np.ndarray:
+    """The ten reward parameters (include/nav3d.h ``nav3d_reward_params``, field order) as float64: the reference's
+    literals with ``crash_penalty``, overridden by the entries of the dict ``reward``."""
+    d = dict(REWARD_DEFAULTS, crash_penalty=crash_penalty)
+    for k, v in (reward or {}).items():
+        if k not in d:
+            raise KeyError(f"unknown reward parameter {k!r}")
+        d[k] = float(v)
+    return np.array([d[k] for k in REWARD_FIELDS], dtype=np.float64)
+
+
+def py_round2(x: float) -> float:
+    """The oracle's restatement of CPython's ``round(x, 2)`` (simpleEnv distances)."""
+    return lib().orc_py_round2(float(x))
 
 
 class OracleRoom:
@@ -88,12 +112,27 @@ CUBIC_STATE = ("x", "y", "z", "facing", "visited_count", "bump_count", "step_cou
 
 
 class OracleCubic:
-    """One CubicEnv ``GridAgent`` (reference ``envs/CubicEnv.py``) with injected (room, start) picks."""
+    """One CubicEnv ``GridAgent`` (reference ``envs/CubicEnv.py``) with injected (room, start) picks.  ``reward``: a dict
+    of ``nav3d_reward_params`` fields that replace the reference's literals (``reward_values``)."""
 
-    def __init__(self, L: int = 4, crash_penalty: float = -2.0):
+    def __init__(self, L: int = 4, crash_penalty: float = -2.0, reward=None):
         self.L = L
         self.h = lib().orc_cubic_create(L, crash_penalty)
         self.room = None
+        if reward is not None:
+            self.set_reward(reward, crash_penalty)
+
+    def set_reward(self, reward=None, crash_penalty: float = -2.0):
+        self._rw = reward_values(reward, crash_penalty)
+        lib().orc_cubic_set_reward(self.h, _p(self._rw))
+
+    def ret_centi(self) -> int:
+        """The running episode return in 1/100 units (nav3d_get_state column 15)."""
+        return int(lib().orc_cubic_ret_centi(self.h))
+
+    def episode_return(self) -> float:
+        """nav3d_episode.episode_return for the episode so far (f32)."""
+        return float(lib().orc_cubic_episode_return(self.h))
 
     def reset(self, room: OracleRoom, start) -> np.ndarray:
         self.room = room
@@ -247,11 +286,14 @@ class OracleVec:
     """N CubicEnv oracles + the SB3-VecEnv auto-reset contract + Philox picks (mirrors ``nav3d.BatchedCubicEnv``)."""
 
     def __init__(self, n: int, rooms, L: int = 4, crash_penalty: float = -2.0, seed: int = 0, env_id0: int = 0,
-                 auto_reset: bool = True):
+                 auto_reset: bool = True, reward=None):
         self.n = n
         self.rooms = list(rooms)
+        self.crash_penalty = crash_penalty
         arr = (C.c_void_p * len(self.rooms))(*[r.h for r in self.rooms])
         self.h = lib().orc_vec_create(n, len(self.rooms), arr, L, crash_penalty, seed, env_id0, int(auto_reset))
+        if reward is not None:
+            self.set_reward(reward)
         self.obs = np.zeros((n, 80), dtype=np.float32)
         self.reward = np.zeros(n, dtype=np.float64)
         self.terminated = np.zeros(n, dtype=np.uint8)
@@ -261,6 +303,19 @@ class OracleVec:
         self.ep_len = np.zeros(n, dtype=np.int64)
         self.ep_bumps = np.zeros(n, dtype=np.int64)
         self.ep_visited = np.zeros(n, dtype=np.int64)
+        self.ep_ret32 = np.zeros(n, dtype=np.float32)
+
+    def set_reward(self, reward=None):
+        """Replace the reward literals of every env from the next step on (a dict of ``nav3d_reward_params`` fields;
+        unnamed fields take the reference's values and the vec's crash penalty)."""
+        self._rw = reward_values(reward, self.crash_penalty)
+        lib().orc_vec_set_reward(self.h, _p(self._rw))
+
+    def ret_centi(self) -> np.ndarray:
+        """int64 [n]: each env's running episode return in 1/100 units (nav3d_get_state column 15)."""
+        out = np.zeros(self.n, dtype=np.int64)
+        lib().orc_vec_ret_centi(self.h, _p(out))
+        return out
 
     def reset(self, picks=None) -> np.ndarray:
         if picks is not None:
@@ -273,6 +328,7 @@ class OracleVec:
         lib().orc_vec_step(self.h, _p(a), _p(self.obs), _p(self.reward), _p(self.terminated), _p(self.truncated),
                            _p(self.terminal_obs), _p(self.ep_ret), _p(self.ep_len), _p(self.ep_bumps),
                            _p(self.ep_visited))
+        lib().orc_vec_ep_return32(self.h, _p(self.ep_ret32))
         return self.obs, self.reward, self.terminated, self.truncated
 
     def rollout_random(self, T: int, t0: int = 0):

@@ -87,7 +87,7 @@ extern "C" {
 
 void *emu_create(int n_envs, int L, double crash, unsigned long long seed, unsigned env_id0, int auto_reset, int n_rooms,
                  const int *dims, const int8_t *dense, const unsigned *dense_off, int wall_code, int simple, double cell_size,
-                 int lanes, int descending) {
+                 int lanes, int descending, const double *reward /* the ten nav3d_reward_params fields, NULL = reference */) {
     Emu *e = new Emu();
     e->simple = simple != 0;
     e->G = lanes; e->descending = descending != 0;
@@ -128,7 +128,7 @@ void *emu_create(int n_envs, int L, double crash, unsigned long long seed, unsig
     }
     size_t ovf_off = (max_k + 127) / 128 * 128, stride = ovf_off + (max_cells + 127) / 128 * 128;
     if (e->simple) { ovf_off = 0; stride = (max_k + 127) / 128 * 128; }
-    for (int c = 0; c <= L; c++) e->dist_lut.push_back((float)(std::nearbyint((double)c * cell_size * 100.0) / 100.0));
+    for (int c = 0; c <= L; c++) e->dist_lut.push_back((float)py_round2((double)c * cell_size));
     e->states.assign((size_t)n_envs, EnvState{});
     e->know.assign(stride * (size_t)n_envs, 0xAB);     // poison: a reset must clear what it uses
 #ifdef NAV3D_EMU_ASAN
@@ -145,10 +145,14 @@ void *emu_create(int n_envs, int L, double crash, unsigned long long seed, unsig
     P.rooms = e->rooms.data(); P.occz = e->occz.data(); P.occ64 = e->occ64.data(); P.free_cells = e->free_cells.data();
     P.states = e->states.data(); P.know = e->know.data(); P.env_stride = stride; P.ovf_off = (uint32_t)ovf_off;
     P.n_envs = n_envs; P.n_rooms = n_rooms; P.L = L; P.env_id0 = env_id0; P.seed_lo = (uint32_t)seed;
-    P.seed_hi = (uint32_t)(seed >> 32); P.auto_reset = auto_reset; P.rw = reference_reward_params(crash);
+    P.seed_hi = (uint32_t)(seed >> 32); P.auto_reset = auto_reset;
+    P.rw = reward ? reward_params_from(reward) : reference_reward_params(crash);
     P.dist_lut = e->dist_lut.data(); P.obs_dim = e->simple ? 6 * L + 7 : kObsDim;
     return e;
 }
+// the engine's rule for nav3d_set_reward_params (NULL = accepted) and its simpleEnv distance rounding
+const char *emu_reward_params_reject(const double *reward) { return reward_params_reject(reward_params_from(reward)); }
+double emu_py_round2(double x) { return py_round2(x); }
 void emu_destroy(void *h) {
 #ifdef NAV3D_EMU_ASAN
     ASAN_UNPOISON_MEMORY_REGION(((Emu *)h)->know.data(), ((Emu *)h)->know.size());

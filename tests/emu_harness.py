@@ -34,7 +34,11 @@ def lib():
         L = C.CDLL(str(LIB))
         P, I = C.c_void_p, C.c_int
         L.emu_create.restype = P
-        L.emu_create.argtypes = [I, I, C.c_double, C.c_uint64, C.c_uint32, I, I, P, P, P, I, I, C.c_double, I, I]
+        L.emu_create.argtypes = [I, I, C.c_double, C.c_uint64, C.c_uint32, I, I, P, P, P, I, I, C.c_double, I, I, P]
+        L.emu_reward_params_reject.restype = C.c_char_p
+        L.emu_reward_params_reject.argtypes = [P]
+        L.emu_py_round2.restype = C.c_double
+        L.emu_py_round2.argtypes = [C.c_double]
         L.emu_destroy.argtypes = [P]
         L.emu_room_n_free.restype = I
         L.emu_room_n_free.argtypes = [P, I]
@@ -52,7 +56,9 @@ def _p(a):
 
 class EmuEngine:
     def __init__(self, n, rooms, L=4, crash_penalty=-2.0, seed=0, env_id0=0, auto_reset=True, simple=False, cell_size=0.25,
-                 lanes=1, descending=False):
+                 lanes=1, descending=False, reward=None):
+        """``reward``: the ten ``nav3d_reward_params`` values in field order (``oracle.c_oracle.reward_values``) or None for
+        the reference's literals with ``crash_penalty``."""
         self.n = n
         self.obs_dim = 6 * L + 7 if simple else 80
         self.rooms = rooms
@@ -63,8 +69,11 @@ class EmuEngine:
             offs[i] = o
             o += r.grid.size
         dense = np.concatenate([np.ascontiguousarray(r.grid, dtype=np.int8).ravel() for r in rooms])
+        rw = None if reward is None else np.ascontiguousarray(reward, dtype=np.float64)
+        assert rw is None or rw.shape == (10,)
         self.h = lib().emu_create(n, L, crash_penalty, seed, env_id0, int(auto_reset), len(rooms), _p(dims), _p(dense),
-                                  _p(offs), int(rooms[0].wall_code), int(simple), cell_size, int(lanes), int(descending))
+                                  _p(offs), int(rooms[0].wall_code), int(simple), cell_size, int(lanes), int(descending),
+                                  _p(rw))
         self.obs = np.zeros((n, self.obs_dim), np.float32)
         self.reward = np.zeros(n, np.float32)
         self.reward64 = np.zeros(n, np.float64)

@@ -123,12 +123,17 @@ class _Rows:
     """The rows `r` of an oracle vector, with the attribute names lockstep.compare_step reads."""
 
     def __init__(self, ov, r):
-        for k in ("obs", "reward", "terminated", "truncated", "terminal_obs", "ep_ret", "ep_len", "ep_bumps", "ep_visited"):
+        for k in ("obs", "reward", "terminated", "truncated", "terminal_obs", "ep_ret", "ep_len", "ep_bumps", "ep_visited",
+                  "ep_ret32"):
             setattr(self, k, getattr(ov, k)[r])
         self._state = ov.state()[r]
+        self._ret_centi = ov.ret_centi()[r]
 
     def state(self):
         return self._state
+
+    def ret_centi(self):
+        return self._ret_centi
 
 
 def _oracle_step(ov, e, t, actions, r):

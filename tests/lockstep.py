@@ -3,6 +3,12 @@ next to ``oracle.c_oracle.OracleVec`` on identical actions; every output is comp
 import numpy as np
 
 
+def episode_return_bound(length, ret):
+    """include/nav3d.h's bound on |episode_return - sum of the episode's f64 rewards|: 0.005 per rounded term (at most
+    five a step plus the finish and truncation terms), the f32 rounding of the result, and 1e-3 of f64 rounding."""
+    return 0.005 * (5 * np.asarray(length, np.float64) + 2) + 2.0 ** -24 * np.abs(ret) + 1e-3
+
+
 def compare_step(tag, t, ov, obs, reward, reward64, term, trunc, tobs, eps, state, crash_penalty=-2.0):
     done = (ov.terminated | ov.truncated).astype(bool)
     assert np.array_equal(term, ov.terminated), f"{tag} t={t}: terminated differs at {np.nonzero(term != ov.terminated)[0][:8]}"
@@ -25,7 +31,11 @@ def compare_step(tag, t, ov, obs, reward, reward64, term, trunc, tobs, eps, stat
             assert np.array_equal(e[:, 2], ov.ep_bumps[done]), f"{tag} t={t}: episode bumps"
             assert np.array_equal(e[:, 3], ov.ep_visited[done]), f"{tag} t={t}: episode visited"
             ret = e[:, 0].copy().view(np.float32)
-            assert np.allclose(ret, ov.ep_ret[done], rtol=1e-6, atol=1e-4), f"{tag} t={t}: episode return {ret} vs {ov.ep_ret[done]}"
+            want = ov.ep_ret32[done]
+            assert np.array_equal(ret.view(np.uint32), want.view(np.uint32)), f"{tag} t={t}: episode return {ret} vs {want}"
+            err = np.abs(ret.astype(np.float64) - ov.ep_ret[done])
+            assert (err <= episode_return_bound(ov.ep_len[done], ov.ep_ret[done])).all(), \
+                f"{tag} t={t}: episode return {ret} is {err.max()} from the f64 sum {ov.ep_ret[done]}"
             assert np.array_equal(e[:, 6], ov.terminated[done]) and np.array_equal(e[:, 7], ov.truncated[done])
     if state is not None:
         os_ = ov.state()
@@ -35,6 +45,11 @@ def compare_step(tag, t, ov, obs, reward, reward64, term, trunc, tobs, eps, stat
         if len(bad):
             i = bad[0]
             raise AssertionError(f"{tag} t={t}: state differs for {len(bad)} envs; env {i} got {got[i]} want {os_[i]}")
+        if state.shape[1] > 15:
+            rc = ov.ret_centi()
+            bad = np.nonzero(state[:, 15].astype(np.int64) != rc)[0]
+            assert not len(bad), f"{tag} t={t}: return so far (state[15]) differs for {len(bad)} envs; env {bad[0]} " \
+                                 f"got {state[bad[0], 15]} want {rc[bad[0]]}"
 
 
 def compare_grids(tag, ov, grid_fn, envs):

@@ -1,6 +1,7 @@
 """Parity tests proper: the CUDA path (through the C ABI) against the CPU oracle and the reference's golden traces.
-Integer state, flags, observations (f32) and rewards (f64 and f32) are compared BIT-EXACTLY; the only tolerance is on the
-per-episode return (an f32 summary; 1e-6 relative), stated where it is used (tests/lockstep.py)."""
+Integer state, flags, observations (f32), rewards (f64 and f32) and the per-episode return (the documented 1/100-unit
+rule, restated by the oracle) are compared BIT-EXACTLY; the return is also held to the documented bound against the f64
+sum of the rewards (tests/lockstep.py)."""
 import numpy as np
 import pytest
 
