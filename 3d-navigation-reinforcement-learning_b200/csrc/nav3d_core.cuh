@@ -155,6 +155,10 @@ struct EngineParams {
     const unsigned long long *occ64;
     const uint32_t *free_cells;
     const uint32_t *room_start;    // per room: x | y<<8 | z<<16 of the file's "Start position" or 0xffffffff (may be null)
+    // Room-draw table of the Philox resets (draw_room): cdf[j] for j < n_rooms, cdf[n_rooms-1] = 2^32.  A fixed device
+    // address for the engine's lifetime with its rooms, rewritten in place by nav3d_set_room_weights, so captured graphs
+    // read the current table.  Read only after griddepcontrol.wait in the programmatically serialised kernels.
+    const unsigned long long *cdf;
     EnvState *states;
     uint8_t *know;                 // per-env knowledge storage: [K bricks | overflow bytes]
     unsigned long long env_stride; // bytes per env in `know`
@@ -319,6 +323,53 @@ NAV3D_HD void philox4x32_10_4(uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3
     o[0] = c0; o[1] = c1; o[2] = c2; o[3] = c3;
 }
 NAV3D_HD uint32_t mulhi_range(uint32_t u, uint32_t n) { return (uint32_t)(((unsigned long long)u * n) >> 32); }
+
+// ---------------------------------------------------------------------------------------------------------------
+// room draw of a Philox reset (include/nav3d.h "Random streams", nav3d_set_room_weights).  The engine holds a table of
+// cumulative thresholds cdf[0 .. n-1], nondecreasing, cdf[n-1] = 2^32; word 0 of the reset block picks
+//     room = #{ j < n - 1 : cdf[j] <= u }          so  P(room = j) = (cdf[j] - cdf[j-1]) / 2^32 exactly.
+// The uniform table cdf[j] = ceil((j + 1) 2^32 / n) makes this (u * n) >> 32 for every u: r 2^32 <= u n < (r+1) 2^32
+// <=> ceil(r 2^32 / n) <= u < ceil((r+1) 2^32 / n) for an integer u.
+// ---------------------------------------------------------------------------------------------------------------
+constexpr unsigned long long kCdfOne = 1ull << 32;
+
+// Upper-bound binary search; cdf[n-1] is never read (it is 2^32 > u).  ceil(log2 n) <= 16 probes for n <= 65535.
+// The engine always has a table (nav3d_load_rooms allocates it), so device code has this one path.  A host build of this
+// source that installs no table (the host emulation of tests/emu) gets (u * n) >> 32, which the uniform table reproduces.
+NAV3D_HD uint32_t draw_room(const unsigned long long *cdf, uint32_t n, uint32_t u) {
+#ifndef __CUDA_ARCH__
+    if (cdf == nullptr) return mulhi_range(u, n);
+#endif
+    uint32_t lo = 0, hi = n - 1u;
+    while (lo < hi) {
+        const uint32_t mid = (lo + hi) >> 1;
+        if (ldg(cdf + mid) <= (unsigned long long)u) lo = mid + 1u; else hi = mid;
+    }
+    return lo;
+}
+NAV3D_HD unsigned long long room_cdf_uniform(uint32_t j, uint32_t n) {
+    return (((unsigned long long)(j + 1u) << 32) + n - 1u) / n;
+}
+// Table from f32 weights w (nav3d_set_room_weights), in integer / IEEE steps of fixed order so that a reference restates it
+// bit for bit, whatever order a builder visits the rooms in:
+//   q_j = floor(fl(w_j / w_max) * 2^32)            (one correctly rounded f64 division; the scaling is exact), q_max = 2^32
+//   C_j = q_0 + ... + q_j  (u64, < 2^48)           cdf[j] = ceil(2^32 C_j / C_{n-1})  (128-bit)
+// A weight is accepted if it is finite and not negative (-0 counts as 0); a vector needs one positive weight.
+NAV3D_HD bool room_weight_ok(float w) { return w >= 0.0f && w <= 3.402823466e38f; }
+// bits of an accepted weight, ordered as the weight (the max reduction runs on them); -0 -> 0
+NAV3D_HD uint32_t room_weight_bits(float w) { return w > 0.0f ? float_bits(w) : 0u; }
+NAV3D_HD unsigned long long room_weight_q(float w, float w_max) {
+#ifdef __CUDA_ARCH__
+    const double r = __ddiv_rn((double)w, (double)w_max);
+#else
+    const double r = (double)w / (double)w_max;
+#endif
+    return (unsigned long long)(r * 4294967296.0);          // r in [0, 1]: exact scaling, truncation = floor
+}
+NAV3D_HD unsigned long long room_cdf_entry(unsigned long long c, unsigned long long total) {
+    const unsigned __int128 num = ((unsigned __int128)c << 32) + (total - 1u);
+    return (unsigned long long)(num / total);
+}
 
 // ---------------------------------------------------------------------------------------------------------------
 // knowledge-storage addressing (CubicEnv).  Bordered coordinates xp = x + kPadLo, yp = y + kPadLo.
@@ -796,7 +847,7 @@ NAV3D_HD void reset_env(const EngineParams &P, int env, int lane, int lane_in_wa
 NAV3D_HD void reset_picks(const EngineParams &P, int env, uint32_t episode, uint32_t &room, uint32_t &k) {
     uint32_t u0, u1;
     philox4x32_10(P.env_id0 + (uint32_t)env, episode, 0u, kStreamReset, P.seed_lo, P.seed_hi, u0, u1);
-    room = mulhi_range(u0, (uint32_t)P.n_rooms);                      // random.choice(self.rooms) (:407)
+    room = draw_room(P.cdf, (uint32_t)P.n_rooms, u0);                 // random.choice(self.rooms) (:407), weighted
     k = mulhi_range(u1, ldg(&P.rooms[room].n_free));                  // random.choice(possible_start_pose) (:462)
 }
 
@@ -1166,7 +1217,7 @@ NAV3D_HD void simple_reset_env_philox(const EngineParams &P, int env, int lane, 
                                       float *obs_row) {
     uint32_t u[4];
     philox4x32_10_4(P.env_id0 + (uint32_t)env, episode, 0u, kStreamReset, P.seed_lo, P.seed_hi, u);
-    const uint32_t room = mulhi_range(u[0], (uint32_t)P.n_rooms);                 // random.choice(self.rooms) (:351)
+    const uint32_t room = draw_room(P.cdf, (uint32_t)P.n_rooms, u[0]);            // random.choice(self.rooms) (:351), weighted
     const uint32_t nf = ldg(&P.rooms[room].n_free);
     simple_reset_env<G>(P, env, lane, lane_in_warp, room, mulhi_range(u[1], nf), mulhi_range(u[2], nf), episode + 1u, obs_row);
 }

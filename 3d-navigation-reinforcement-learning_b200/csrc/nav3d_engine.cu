@@ -647,6 +647,71 @@ __global__ void __launch_bounds__(kBlock) load_envs_kernel(const __grid_constant
     if (st == kBlobLoaded) load_env_lane(P, env, blob, obs, lane, 32);
 }
 
+// nav3d_set_room_weights: the room-draw table from f32 weights (nav3d_core.cuh room_weight_q / room_cdf_entry), or the
+// uniform table when w is null.  One CTA: validate and reduce w_max, then a block-wide scan of the q_j over contiguous
+// chunks, then the write.  A rejected vector returns before anything is written.
+constexpr int kCdfThreads = 1024;
+__global__ void __launch_bounds__(kCdfThreads) room_cdf_kernel(const float *__restrict__ w, int n,
+                                                               unsigned long long *cdf, uint8_t *status) {
+    __shared__ uint32_t wmax;
+    __shared__ unsigned long long warp_sum[kCdfThreads / 32], grand;
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    if (w == nullptr) {
+        for (int j = tid; j < n; j += kCdfThreads) cdf[j] = room_cdf_uniform((uint32_t)j, (uint32_t)n);
+        if (status && tid == 0) *status = 0;
+        return;
+    }
+    const int chunk = (n + kCdfThreads - 1) / kCdfThreads;
+    const int lo = min(n, tid * chunk), hi = min(n, lo + chunk);
+    if (tid == 0) wmax = 0u;
+    bool bad = false;
+    uint32_t mx = 0u;
+    for (int j = lo; j < hi; j++) {
+        const float v = w[j];
+        bad |= !room_weight_ok(v);
+        mx = max(mx, room_weight_bits(v));
+    }
+    mx = __reduce_max_sync(0xffffffffu, mx);
+    __syncthreads();                                        // wmax = 0 is visible
+    if (lane == 0) atomicMax(&wmax, mx);
+    bad = __syncthreads_or(bad);                            // also orders the atomicMax before the read below
+    if (bad || wmax == 0u) {
+        if (status && tid == 0) *status = 1;
+        return;
+    }
+    const float w_max = __uint_as_float(wmax);
+    unsigned long long s = 0;
+    for (int j = lo; j < hi; j++) s += room_weight_q(w[j], w_max);
+    // inclusive scan over the block: within warps, then over the warp totals
+    unsigned long long incl = s;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        const unsigned long long t = __shfl_up_sync(0xffffffffu, incl, o);
+        if (lane >= o) incl += t;
+    }
+    if (lane == 31) warp_sum[warp] = incl;
+    __syncthreads();
+    if (warp == 0) {
+        const unsigned long long t = warp_sum[lane];
+        unsigned long long x = t;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            const unsigned long long y = __shfl_up_sync(0xffffffffu, x, o);
+            if (lane >= o) x += y;
+        }
+        warp_sum[lane] = x - t;                             // exclusive prefix of warp `lane`
+        if (lane == 31) grand = x;                          // C_{n-1}
+    }
+    __syncthreads();
+    const unsigned long long C_total = grand;
+    unsigned long long c = warp_sum[warp] + incl - s;      // C of the element before this thread's chunk
+    for (int j = lo; j < hi; j++) {
+        c += room_weight_q(w[j], w_max);
+        cdf[j] = room_cdf_entry(c, C_total);
+    }
+    if (status && tid == 0) *status = 0;
+}
+
 size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
 }  // namespace
@@ -665,6 +730,7 @@ struct nav3d_engine {
     uint16_t *d_occz = nullptr;
     unsigned long long *d_occ64 = nullptr;
     uint32_t *d_free = nullptr, *d_start = nullptr;
+    unsigned long long *d_cdf = nullptr;   // room-draw table (EngineParams::cdf), allocated with the rooms
     EnvState *d_states = nullptr;
     uint8_t *d_know = nullptr;
     size_t know_bytes = 0, room_bytes = 0;
@@ -705,6 +771,7 @@ struct DeviceGuard {
 void free_rooms(nav3d_engine *e) {
     cudaFree(e->d_rooms); cudaFree(e->d_occz); cudaFree(e->d_occ64); cudaFree(e->d_free); cudaFree(e->d_know);
     cudaFree(e->d_start); e->d_start = nullptr;
+    cudaFree(e->d_cdf); e->d_cdf = nullptr;
     e->d_rooms = nullptr; e->d_occz = nullptr; e->d_occ64 = nullptr; e->d_free = nullptr; e->d_know = nullptr;
     e->know_bytes = 0; e->room_bytes = 0;
     e->h_rooms.clear(); e->h_free.clear(); e->h_nwall.clear();
@@ -926,6 +993,12 @@ int nav3d_load_rooms(nav3d_engine *e, int32_t n_rooms, const nav3d_room_desc *ro
     LOAD_TRY(cudaMalloc(&e->d_know, know_bytes));
     LOAD_TRY(cudaMalloc(&e->d_start, sizeof(uint32_t) * n_rooms));
     LOAD_TRY(cudaMemcpy(e->d_start, start.data(), sizeof(uint32_t) * n_rooms, cudaMemcpyHostToDevice));
+    {   // the uniform room-draw table, uploaded with the rooms (no launch): resets draw (u * n_rooms) >> 32 as before
+        std::vector<unsigned long long> cdf((size_t)n_rooms);
+        for (int j = 0; j < n_rooms; j++) cdf[(size_t)j] = room_cdf_uniform((uint32_t)j, (uint32_t)n_rooms);
+        LOAD_TRY(cudaMalloc(&e->d_cdf, sizeof(unsigned long long) * n_rooms));
+        LOAD_TRY(cudaMemcpy(e->d_cdf, cdf.data(), sizeof(unsigned long long) * n_rooms, cudaMemcpyHostToDevice));
+    }
     LOAD_TRY(cudaMemcpy(d_dense, dense.data(), n_dense, cudaMemcpyHostToDevice));
     LOAD_TRY(cudaMemcpy(d_off, dense_off.data(), sizeof(uint32_t) * n_rooms, cudaMemcpyHostToDevice));
     LOAD_TRY(cudaMemcpy(d_wall, wall.data(), sizeof(int32_t) * n_rooms, cudaMemcpyHostToDevice));
@@ -956,11 +1029,11 @@ int nav3d_load_rooms(nav3d_engine *e, int32_t n_rooms, const nav3d_room_desc *ro
     for (int i = 0; i < n_rooms; i++)
         e->signature = sig_room(e->signature, rooms[i].width, rooms[i].depth, rooms[i].height, rooms[i].wall_code,
                                 rooms[i].grid, start[(size_t)i]);
-    e->room_bytes = sizeof(RoomDev) * n_rooms + 2 * n_occz + 8 * n_occ64 + 4 * n_free_cap;
+    e->room_bytes = sizeof(RoomDev) * n_rooms + 2 * n_occz + 8 * n_occ64 + 4 * n_free_cap + 8 * (size_t)n_rooms;
     EngineParams &P = e->P;
     P.rooms = e->d_rooms; P.occz = e->d_occz; P.occ64 = e->d_occ64; P.free_cells = e->d_free;
     P.know = e->d_know; P.env_stride = stride; P.ovf_off = (uint32_t)ovf_off; P.n_rooms = n_rooms;
-    P.room_start = e->d_start;
+    P.room_start = e->d_start; P.cdf = e->d_cdf;
     e->reset_seen = false;
     return NAV3D_OK;
 }
@@ -983,6 +1056,26 @@ int nav3d_set_reward_params(nav3d_engine *e, const nav3d_reward_params *p) {
     const RewardParams w = reward_params_from(v);
     if (const char *why = reward_params_reject(w)) return fail(NAV3D_ERR_UNSUPPORTED, std::string("nav3d_set_reward_params: ") + why);
     e->P.rw = w;
+    return NAV3D_OK;
+}
+
+int nav3d_set_room_weights(nav3d_engine *e, const float *weights, uint8_t *status, void *stream) {
+    if (int rc = check_ready(e)) return rc;
+    NAV3D_DEVICE(e);
+    // launched without programmatic stream serialisation: it starts only after the previous kernel of the stream (a step
+    // that may still be drawing rooms from the table) has finished
+    room_cdf_kernel<<<1, kCdfThreads, 0, (cudaStream_t)stream>>>(weights, (int)e->h_rooms.size(), e->d_cdf, status);
+    e->launches++;
+    CUDA_TRY(cudaGetLastError());
+    return NAV3D_OK;
+}
+
+int nav3d_get_room_cdf(nav3d_engine *e, uint64_t *cdf, void *stream) {
+    if (int rc = check_ready(e)) return rc;
+    if (!cdf) return fail(NAV3D_ERR_INVALID, "cdf is NULL");
+    NAV3D_DEVICE(e);
+    CUDA_TRY(cudaMemcpyAsync(cdf, e->d_cdf, sizeof(unsigned long long) * e->h_rooms.size(), cudaMemcpyDeviceToDevice,
+                             (cudaStream_t)stream));
     return NAV3D_OK;
 }
 

@@ -58,6 +58,8 @@ SYMBOLS = {
     "nav3d_destroy": (None, [_P]),
     "nav3d_reward_params_default": (None, [C.POINTER(RewardParams)]),
     "nav3d_set_reward_params": (C.c_int, [_P, C.POINTER(RewardParams)]),
+    "nav3d_set_room_weights": (C.c_int, [_P, _P, _P, _P]),
+    "nav3d_get_room_cdf": (C.c_int, [_P, _P, _P]),
     "nav3d_load_rooms": (C.c_int, [_P, C.c_int32, C.POINTER(RoomDesc)]),
     "nav3d_room_info": (C.c_int, [_P, C.c_int32, C.POINTER(C.c_int32)]),
     "nav3d_room_free_cell": (C.c_int, [_P, C.c_int32, C.c_int32, C.POINTER(C.c_int32)]),

@@ -100,6 +100,45 @@ class Engine:
         self.reward_params = {f: float(getattr(p, f)) for f, _ in _lib.RewardParams._fields_}
         self.crash_penalty = self.reward_params["crash_penalty"]
 
+    def set_room_weights(self, weights=None, *, check: bool = True):
+        """Draw the rooms of every later Philox reset (``reset`` without picks, auto-resets, rollouts) with probability
+        proportional to ``weights`` (include/nav3d.h ``nav3d_set_room_weights``); None restores the uniform draw.
+
+        ``weights``: a 1-D sequence, NumPy array or tensor of ``len(rooms)`` non-negative finite values, not all zero; it
+        becomes a contiguous float32 tensor on the engine's device (a tensor that already is one is used in place).  One
+        kernel launch on the current stream.  ``check=True`` reads the status back (one synchronisation) and raises
+        ``Nav3dError`` naming why a vector was rejected; ``check=False`` synchronises nothing and can be captured in a CUDA
+        graph, and a rejected vector then silently leaves the table as it was."""
+        n = len(self.rooms)
+        w = None
+        if weights is not None:
+            w = weights if isinstance(weights, torch.Tensor) else torch.as_tensor(np.asarray(weights, dtype=np.float32))
+            if w.dim() != 1 or w.numel() != n:
+                raise ValueError(f"weights must be a 1-D sequence of {n} values (one per room), got shape {tuple(w.shape)}")
+            w = w.to(device=self.device, dtype=torch.float32).contiguous()
+        status = torch.empty(1, dtype=torch.uint8, device=self.device) if check and w is not None else None
+        with torch.cuda.device(self.device):
+            _lib.check(self._lib.nav3d_set_room_weights(self._h, _ptr(w), _ptr(status), self._stream()))
+        if status is not None and int(status.item()) != 0:
+            h = w.cpu().numpy()
+            why = ("NaN at rooms " + str(np.nonzero(np.isnan(h))[0][:16].tolist()) if np.isnan(h).any() else
+                   "infinite value at rooms " + str(np.nonzero(np.isinf(h))[0][:16].tolist()) if np.isinf(h).any() else
+                   "negative value at rooms " + str(np.nonzero(h < 0)[0][:16].tolist()) if (h < 0).any() else
+                   "all weights are 0")
+            raise Nav3dError(-1, f"set_room_weights: {why}; the room table is unchanged")
+
+    def room_cdf(self) -> torch.Tensor:
+        """The room-draw table (``nav3d_get_room_cdf``) as int64 [n_rooms] on the engine's device; the last entry is 2^32."""
+        out = torch.empty(len(self.rooms), dtype=torch.int64, device=self.device)
+        with torch.cuda.device(self.device):
+            check(self._lib.nav3d_get_room_cdf(self._h, _ptr(out), self._stream()))
+        return out
+
+    def room_probabilities(self) -> torch.Tensor:
+        """float64 [n_rooms]: the exact probability of each room in a Philox reset, diff(cdf) / 2^32.  A positive weight
+        below max(weights) * 2^-32 shows here as 0, as it is drawn."""
+        return torch.diff(self.room_cdf(), prepend=torch.zeros(1, dtype=torch.int64, device=self.device)).double() / 2.0 ** 32
+
     def free_cell(self, room: int, k: int):
         xyz = (C.c_int32 * 3)()
         check(self._lib.nav3d_room_free_cell(self._h, int(room), int(k), xyz))

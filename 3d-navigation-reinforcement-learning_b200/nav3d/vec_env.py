@@ -172,6 +172,14 @@ class BatchedCubicEnv:
     def state(self) -> torch.Tensor:
         return self.engine.get_state()
 
+    def set_room_weights(self, weights=None, *, check: bool = True) -> None:
+        """Weighted room draw for every later reset (``Engine.set_room_weights``); None = uniform."""
+        self.engine.set_room_weights(weights, check=check)
+
+    def room_probabilities(self) -> torch.Tensor:
+        """float64 [n_rooms]: each room's exact probability in a reset (``Engine.room_probabilities``)."""
+        return self.engine.room_probabilities()
+
     def save_envs(self, indices, obs: Optional[torch.Tensor] = None) -> torch.Tensor:
         """Complete state of the listed envs as uint8 [n, engine.env_state_bytes] device blobs (``Engine.save_envs``).
         ``obs`` is the current observation array: this env's own buffer by default; pass the tensor the last
@@ -281,6 +289,14 @@ class BatchedSimpleEnv:
     def step(self, actions):
         self.step_async(actions)
         return self.step_wait()
+
+    def set_room_weights(self, weights=None, *, check: bool = True) -> None:
+        """Weighted room draw for every later reset (``Engine.set_room_weights``); None = uniform."""
+        self.engine.set_room_weights(weights, check=check)
+
+    def room_probabilities(self) -> torch.Tensor:
+        """float64 [n_rooms]: each room's exact probability in a reset (``Engine.room_probabilities``)."""
+        return self.engine.room_probabilities()
 
     def save_envs(self, indices, obs: Optional[torch.Tensor] = None) -> torch.Tensor:
         """As ``BatchedCubicEnv.save_envs``."""

@@ -21,11 +21,14 @@
  *
  * Random streams (counter-based Philox4x32-10, Salmon et al. SC'11) — documented because the oracle restates them:
  *   key = (seed & 0xffffffff, seed >> 32);  counter = (global_env_id, index, 0, stream_tag)
- *   stream_tag 0x52455345: index = episode number of that env (0 for the first reset); output word 0 -> room index,
- *                          word 1 -> index k into the room's list of free interior cells (x-major, then y, then z —
- *                          the order envs/CubicEnv.py:450-457 builds possible_start_pose in)
+ *   stream_tag 0x52455345: index = episode number of that env (0 for the first reset); output word 0 -> room index
+ *                          through the engine's room-draw table (nav3d_set_room_weights): room = #{ j < n_rooms - 1 :
+ *                          cdf[j] <= word0 }; the uniform table, which every engine holds until weights are set, makes
+ *                          this (word0 * n_rooms) >> 32.  Word 1 -> index k into the chosen room's list of free interior
+ *                          cells (x-major, then y, then z — the order envs/CubicEnv.py:450-457 builds possible_start_pose
+ *                          in); simpleEnv: word 2 -> the goal's index in the same list
  *   stream_tag 0x41435449: index = rollout step t; output word 0 -> action
- *   a 32-bit word u maps to [0, n) as (u * n) >> 32.
+ *   a 32-bit word u maps to [0, n) as (u * n) >> 32 (every draw but the room).
  *   global_env_id = config.env_id0 + local env index, so results do not depend on how envs are sharded over GPUs.
  */
 #ifndef NAV3D_H
@@ -153,17 +156,52 @@ void nav3d_destroy(nav3d_engine *e);
 void nav3d_reward_params_default(nav3d_reward_params *out);
 /* Takes effect from the next launch on; may be called at any time, mid-episode too (host-side copy, no device work).
  * The parameters are copied into each kernel's launch arguments, so a CUDA graph captured before this call keeps
- * replaying with the values it captured: capture the graph again after changing them.  Env-state blobs hold no reward
+ * replaying with the values it captured: capture the graph again after changing them (the room-draw table of
+ * nav3d_set_room_weights is the opposite: graphs read it at replay).  Env-state blobs hold no reward
  * parameters: a loaded env continues with those of the engine it is loaded into.  CubicEnv only (NAV3D_ERR_UNSUPPORTED
  * for simpleEnv).  The accepted sets are described at nav3d_reward_params. */
 int nav3d_set_reward_params(nav3d_engine *e, const nav3d_reward_params *params);
+
+/* ---- weighted room draw.  Every reset that draws from the Philox stream (nav3d_reset with picks == NULL, the auto-resets
+ * of nav3d_step / nav3d_step_host and of both fused rollouts) picks its room through a per-engine DEVICE table of
+ * cumulative thresholds cdf[0 .. n_rooms-1] (nondecreasing, cdf[n_rooms-1] = 2^32):
+ *     room = #{ j < n_rooms - 1 : cdf[j] <= word0 },   P(room = j) = (cdf[j] - cdf[j-1]) / 2^32 exactly (cdf[-1] = 0).
+ * nav3d_load_rooms installs the uniform table cdf[j] = ceil((j + 1) 2^32 / n_rooms), with which every draw equals the
+ * unweighted (word0 * n_rooms) >> 32.  Only the room changes: the start cell (and simpleEnv's goal) are drawn from the
+ * chosen room by words 1 and 2 as before.
+ *
+ * The table from weights w (f32, W = sum of w, w_max = max of w), in steps of fixed order:
+ *     q_j = floor(fl64(w_j / w_max) * 2^32)    (one correctly rounded f64 division)
+ *     C_j = q_0 + ... + q_j  (exact integers)  cdf[j] = ceil(2^32 * C_j / C_{n-1})
+ *   - a zero weight has probability exactly 0; so has a positive weight below w_max * 2^-32 (q_j = 0), which
+ *     nav3d_get_room_cdf shows;
+ *   - equal positive weights give exactly the uniform table;
+ *   - |P(room = j) - w_j / W| <= (2 + (n_rooms - 1) * w_j / W) * 2^-32 + 2^-52  <=  (n_rooms + 1) * 2^-32 + 2^-52
+ *     (flooring q loses less than one unit per room, which moves at most (n_rooms - 1) units of C between rooms; the two
+ *     ceilings cost less than one unit; the division at most 2^-53 relative);
+ *   - the table depends on the weight vector only, so engines given the same weights (shards with different env_id0, other
+ *     lanes_per_env) draw the same room for the same global env id and episode.
+ *
+ * The table is engine configuration, like the reward parameters: env-state blobs and nav3d_snapshot / nav3d_restore do not
+ * hold it, and a loaded or restored env draws its next room from the table of the engine it is in.  Unlike the reward
+ * parameters, which a CUDA graph captures by value, the table lives at one device address for as long as the rooms are
+ * loaded, so a graph captured before nav3d_set_room_weights replays with the table that is current when it runs. */
+
+/* weights: DEVICE f32[n_rooms] or NULL (= the uniform table); status: DEVICE u8[1] or NULL: 0 installed, 1 rejected (a
+ * value is NaN, +-inf or negative, or all values are 0; the table is left as it was).  One kernel launch on `stream`,
+ * launched without programmatic dependent launch so it starts after the previous kernel of the stream has finished; no
+ * allocation, no synchronisation, no host copy: capturable in a CUDA graph, with device-computed weights too. */
+int nav3d_set_room_weights(nav3d_engine *e, const float *weights, uint8_t *status, void *stream);
+/* DEVICE u64[n_rooms]: the current table cdf[j] as above, cdf[n_rooms-1] = 2^32.  Asynchronous device-to-device copy. */
+int nav3d_get_room_cdf(nav3d_engine *e, uint64_t *cdf, void *stream);
 
 /* The room table: replaces the per-reset text parse + free-cell scan of load_room (envs/CubicEnv.py:402-459).
  * Dense grids are uploaded once; a CUDA kernel packs each room into bit-packed occupancy words (three orientations)
  * and builds the ordered free-cell list; per-env knowledge storage is sized for the largest room.
  * After this call the envs must be reset before they are stepped: nav3d_step / nav3d_step_host / nav3d_rollout_random
  * fail with NAV3D_ERR_INVALID until nav3d_reset has been called (the reference raises AttributeError for step-before-
- * reset); an env that a partial reset left out only bumps in place until it is reset. */
+ * reset); an env that a partial reset left out only bumps in place until it is reset.  Installs the uniform room-draw
+ * table (nav3d_set_room_weights), replacing any weights set before. */
 int nav3d_load_rooms(nav3d_engine *e, int32_t n_rooms, const nav3d_room_desc *rooms);
 /* out6 = width, depth, height, total_free_cells (= max_steps, CubicEnv.py:459), n_wall_cells, reserved.  Synchronises. */
 int nav3d_room_info(nav3d_engine *e, int32_t room, int32_t *out6);
