@@ -712,6 +712,168 @@ __global__ void __launch_bounds__(kCdfThreads) room_cdf_kernel(const float *__re
     if (status && tid == 0) *status = 0;
 }
 
+// nav3d_room_stats: per-room sums of the finished episodes of T x n_envs (step, env) rows.  Each thread owns chunks of 16
+// consecutive rows of the flat flag arrays, placed so that `term` is read with one 16-byte load per chunk (the chunks that
+// straddle the ends of the array are read byte by byte); an all-zero chunk costs its two loads.  Flagged rows load their
+// episode record and go into a per-thread run of equal rooms; a run is flushed when the room changes and at the end of
+// every chunk, where the warp first merges the runs of equal rooms (__match_any_sync, then a tree of shuffles over each
+// group's members).  A flush adds to privatised shared-memory bins when n_rooms <= kStatSmemRooms (bins that received a row
+// are added to `acc` when the CTA ends) and to `acc` with 64-bit atomics otherwise.  All sums are integers: the result does
+// not depend on the order.
+constexpr int kStatThreads = 256;
+constexpr int kStatSmemRooms = 256;
+constexpr int kStatFields = 7;          // nav3d_room_stat fields before `reserved`
+
+struct StatRun {                          // per-thread run of flagged rows of one room
+    uint32_t room, n, term, tl;
+    long long len, bumps, vis, ret;
+};
+
+__device__ __forceinline__ void stat_add(unsigned long long *dst, const StatRun &r) {
+    // dst: the 8 u64 of one room (shared or global); fields that add 0 are skipped
+    atomicAdd(dst + 0, (unsigned long long)r.n);
+    if (r.term) atomicAdd(dst + 1, (unsigned long long)r.term);
+    if (r.tl) atomicAdd(dst + 2, (unsigned long long)r.tl);
+    if (r.len) atomicAdd(dst + 3, (unsigned long long)r.len);
+    if (r.bumps) atomicAdd(dst + 4, (unsigned long long)r.bumps);
+    if (r.vis) atomicAdd(dst + 5, (unsigned long long)r.vis);
+    if (r.ret) atomicAdd(dst + 6, (unsigned long long)r.ret);
+}
+
+template <bool kSmem>
+__global__ void __launch_bounds__(kStatThreads) room_stats_kernel(const uint8_t *__restrict__ term,
+                                                                  const uint8_t *__restrict__ trunc,
+                                                                  const uint8_t *__restrict__ eps, long long M, int n_rooms,
+                                                                  unsigned long long *__restrict__ acc, uint8_t *status) {
+    __shared__ unsigned long long bins[kSmem ? kStatSmemRooms * 8 : 1];
+    __shared__ int block_bad;
+    const int lane = threadIdx.x & 31;
+    if (threadIdx.x == 0) block_bad = 0;
+    if (kSmem)
+        for (int j = threadIdx.x; j < n_rooms * 8; j += kStatThreads) bins[j] = 0ull;
+    __syncthreads();
+    unsigned long long *sink = kSmem ? bins : acc;
+
+    const int a = (int)((uintptr_t)term & 15u);            // chunk c holds rows [16c - a, 16c - a + 16)
+    const bool trunc_vec = (((uintptr_t)trunc - (uintptr_t)term) & 15u) == 0;
+    const bool eps_vec = ((uintptr_t)eps & 15u) == 0;
+    const long long n_chunks = (M + a + 15) / 16;
+    const long long warp0 = ((long long)blockIdx.x * kStatThreads + (threadIdx.x & ~31)), stride = (long long)gridDim.x * kStatThreads;
+    bool bad = false;
+    StatRun run{0u, 0u, 0u, 0u, 0, 0, 0, 0};
+
+    for (long long base = warp0; base < n_chunks; base += stride) {      // warp-uniform trip count
+        const long long c = base + lane;
+        const long long r0 = 16 * c - a;
+        uint32_t tw[4], rw[4];                              // the chunk's 16 flag bytes of each array
+        if (c < n_chunks && r0 >= 0 && r0 + 16 <= M) {
+            const uint4 t4 = __ldg(reinterpret_cast<const uint4 *>(term + r0));
+            tw[0] = t4.x; tw[1] = t4.y; tw[2] = t4.z; tw[3] = t4.w;
+            if (trunc_vec) {
+                const uint4 r4 = __ldg(reinterpret_cast<const uint4 *>(trunc + r0));
+                rw[0] = r4.x; rw[1] = r4.y; rw[2] = r4.z; rw[3] = r4.w;
+            } else {
+#pragma unroll
+                for (int k = 0; k < 4; k++) {
+                    rw[k] = 0u;
+#pragma unroll
+                    for (int b = 0; b < 4; b++) rw[k] |= (uint32_t)__ldg(trunc + r0 + 4 * k + b) << (8 * b);
+                }
+            }
+        } else {
+#pragma unroll
+            for (int k = 0; k < 4; k++) {
+                tw[k] = rw[k] = 0u;
+#pragma unroll
+                for (int b = 0; b < 4; b++) {
+                    const long long r = r0 + 4 * k + b;
+                    if (c < n_chunks && r >= 0 && r < M) {
+                        tw[k] |= (uint32_t)__ldg(term + r) << (8 * b);
+                        rw[k] |= (uint32_t)__ldg(trunc + r) << (8 * b);
+                    }
+                }
+            }
+        }
+        uint32_t tmask = 0u, fmask = 0u;                    // bit j: row r0 + j terminated / flagged
+        if ((tw[0] | tw[1] | tw[2] | tw[3] | rw[0] | rw[1] | rw[2] | rw[3]) != 0u) {
+#pragma unroll
+            for (int j = 0; j < 16; j++) {
+                const uint32_t tb = (tw[j >> 2] >> (8 * (j & 3))) & 0xffu, rb = (rw[j >> 2] >> (8 * (j & 3))) & 0xffu;
+                tmask |= (uint32_t)(tb != 0u) << j;
+                fmask |= (uint32_t)((tb | rb) != 0u) << j;
+            }
+        }
+        while (fmask) {
+            const int j = __ffs(fmask) - 1;
+            fmask &= fmask - 1u;
+            const bool is_term = (tmask >> j) & 1u;
+            const uint8_t *rec = eps + (size_t)(r0 + j) * 32;
+            int ret_bits, len, bumps, vis, room;
+            if (eps_vec) {
+                const int4 v = __ldg(reinterpret_cast<const int4 *>(rec));
+                ret_bits = v.x; len = v.y; bumps = v.z; vis = v.w;
+            } else {
+                ret_bits = __ldg(reinterpret_cast<const int *>(rec));
+                len = __ldg(reinterpret_cast<const int *>(rec) + 1);
+                bumps = __ldg(reinterpret_cast<const int *>(rec) + 2);
+                vis = __ldg(reinterpret_cast<const int *>(rec) + 3);
+            }
+            room = __ldg(reinterpret_cast<const int *>(rec) + 5);
+            const double ret100 = 100.0 * (double)__int_as_float(ret_bits);   // exact: 24 x 7 significant bits
+            if ((uint32_t)room >= (uint32_t)n_rooms || !(fabs(ret100) < 9223372036854775808.0)) {
+                bad = true;                              // also NaN and +-inf
+                continue;
+            }
+            if (run.n && run.room != (uint32_t)room) {
+                stat_add(sink + (size_t)run.room * 8, run);
+                run = StatRun{0u, 0u, 0u, 0u, 0, 0, 0, 0};
+            }
+            run.room = (uint32_t)room;
+            run.n += 1;
+            run.term += is_term;
+            run.tl += !is_term;
+            run.len += len; run.bumps += bumps; run.vis += vis;
+            run.ret += __double2ll_rn(ret100);
+        }
+        // end of chunk: merge the runs of equal rooms across the warp, then each group's first lane flushes
+        const bool has = run.n != 0;
+        if (__any_sync(0xffffffffu, has)) {
+            const unsigned key = has ? run.room : 0xffffffffu;
+            const unsigned grp = __match_any_sync(0xffffffffu, key);
+            const int rank = __popc(grp & ((1u << lane) - 1u)), size = __popc(grp);
+            const int max_size = (int)__reduce_max_sync(0xffffffffu, (unsigned)size);
+            uint32_t cnt = run.n | (run.term << 10) | (run.tl << 20);          // each <= 16 * 32 < 2^10: no carry
+            for (int o = 1; o < max_size; o <<= 1) {                          // tree over the group's ranks
+                const bool take = (rank & (2 * o - 1)) == 0 && rank + o < size;
+                unsigned above = grp & ~((2u << lane) - 1u);                  // members above this lane
+                for (int i = 1; i < o; i++) above &= above - 1u;
+                const int src = take ? __ffs(above) - 1 : lane;               // the member of rank `rank + o`
+                const uint32_t c2 = __shfl_sync(0xffffffffu, cnt, src);
+                const long long l2 = __shfl_sync(0xffffffffu, run.len, src), b2 = __shfl_sync(0xffffffffu, run.bumps, src);
+                const long long v2 = __shfl_sync(0xffffffffu, run.vis, src), e2 = __shfl_sync(0xffffffffu, run.ret, src);
+                if (take) { cnt += c2; run.len += l2; run.bumps += b2; run.vis += v2; run.ret += e2; }
+            }
+            if (has && rank == 0) {
+                run.n = cnt & 0x3ffu; run.term = (cnt >> 10) & 0x3ffu; run.tl = cnt >> 20;
+                stat_add(sink + (size_t)run.room * 8, run);
+            }
+            run = StatRun{0u, 0u, 0u, 0u, 0, 0, 0, 0};
+        }
+    }
+    if (bad) block_bad = 1;
+    __syncthreads();
+    if (kSmem) {
+        for (int r = threadIdx.x; r < n_rooms; r += kStatThreads) {
+            const unsigned long long *b = bins + r * 8;
+            if (b[0] == 0ull) continue;                     // a bin no row reached
+#pragma unroll
+            for (int f = 0; f < kStatFields; f++)
+                if (b[f]) atomicAdd(acc + (size_t)r * 8 + f, b[f]);
+        }
+    }
+    if (status && threadIdx.x == 0 && block_bad) *status = 1;
+}
+
 size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
 }  // namespace
@@ -748,6 +910,7 @@ struct nav3d_engine {
     cudaStream_t copy_stream = nullptr;
     cudaEvent_t chunk_done[kHostChunks] = {};
     uint64_t launches = 0;
+    unsigned stats_grid[2] = {0u, 0u};   // nav3d_room_stats: resident CTAs of room_stats_kernel<false / true> on the device
 };
 
 namespace {
@@ -1076,6 +1239,40 @@ int nav3d_get_room_cdf(nav3d_engine *e, uint64_t *cdf, void *stream) {
     NAV3D_DEVICE(e);
     CUDA_TRY(cudaMemcpyAsync(cdf, e->d_cdf, sizeof(unsigned long long) * e->h_rooms.size(), cudaMemcpyDeviceToDevice,
                              (cudaStream_t)stream));
+    return NAV3D_OK;
+}
+
+int nav3d_room_stats(nav3d_engine *e, int32_t T, const uint8_t *terminated, const uint8_t *truncated,
+                     const nav3d_episode *episodes, nav3d_room_stat *acc, uint8_t *status, void *stream) {
+    if (int rc = check_ready(e)) return rc;
+    if (T < 0) return fail(NAV3D_ERR_INVALID, "T must be >= 0");
+    if (!terminated || !truncated || !episodes || !acc)
+        return fail(NAV3D_ERR_INVALID, "terminated, truncated, episodes and acc are required");
+    if (((uintptr_t)episodes & 3u) || ((uintptr_t)acc & 7u))
+        return fail(NAV3D_ERR_INVALID, "episodes must be 4-byte and acc 8-byte aligned");
+    if (T == 0) return NAV3D_OK;
+    NAV3D_DEVICE(e);
+    const int n_rooms = (int)e->h_rooms.size();
+    const bool smem = n_rooms <= kStatSmemRooms;
+    unsigned &cap = e->stats_grid[smem];
+    if (cap == 0u) {       // one wave of resident CTAs: more would only add shared-bin flushes
+        int sms = 0, per_sm = 0;
+        CUDA_TRY(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, e->cfg.device));
+        CUDA_TRY(smem ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, room_stats_kernel<true>, kStatThreads, 0)
+                      : cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, room_stats_kernel<false>, kStatThreads, 0));
+        cap = (unsigned)std::max(1, sms * std::max(1, per_sm));
+    }
+    const long long M = (long long)T * e->cfg.n_envs;
+    const long long chunks = (M + 15 + 15) / 16;
+    const unsigned grid = (unsigned)std::min<long long>(cap, (chunks + kStatThreads - 1) / kStatThreads);
+    const cudaStream_t s = (cudaStream_t)stream;
+    if (status) CUDA_TRY(cudaMemsetAsync(status, 0, 1, s));
+    auto *out = reinterpret_cast<unsigned long long *>(acc);
+    const auto *eps = reinterpret_cast<const uint8_t *>(episodes);
+    if (smem) room_stats_kernel<true><<<grid, kStatThreads, 0, s>>>(terminated, truncated, eps, M, n_rooms, out, status);
+    else room_stats_kernel<false><<<grid, kStatThreads, 0, s>>>(terminated, truncated, eps, M, n_rooms, out, status);
+    e->launches++;
+    CUDA_TRY(cudaGetLastError());
     return NAV3D_OK;
 }
 

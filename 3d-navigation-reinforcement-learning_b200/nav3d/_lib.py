@@ -49,6 +49,13 @@ class RewardParams(C.Structure):
                                           "truncation_penalty")]
 
 
+class RoomStat(C.Structure):
+    """``nav3d_room_stat``: one room's accumulators of ``nav3d_room_stats`` (64 bytes)."""
+    _fields_ = [("episodes", C.c_uint64), ("terminated", C.c_uint64), ("time_limit", C.c_uint64),
+                ("length_sum", C.c_uint64), ("bumps_sum", C.c_uint64), ("visited_sum", C.c_uint64),
+                ("return_centi_sum", C.c_int64), ("reserved", C.c_uint64)]
+
+
 # every symbol include/nav3d.h declares: (restype, argtypes)
 _P = C.c_void_p
 SYMBOLS = {
@@ -60,6 +67,7 @@ SYMBOLS = {
     "nav3d_set_reward_params": (C.c_int, [_P, C.POINTER(RewardParams)]),
     "nav3d_set_room_weights": (C.c_int, [_P, _P, _P, _P]),
     "nav3d_get_room_cdf": (C.c_int, [_P, _P, _P]),
+    "nav3d_room_stats": (C.c_int, [_P, C.c_int32, _P, _P, _P, _P, _P, _P]),
     "nav3d_load_rooms": (C.c_int, [_P, C.c_int32, C.POINTER(RoomDesc)]),
     "nav3d_room_info": (C.c_int, [_P, C.c_int32, C.POINTER(C.c_int32)]),
     "nav3d_room_free_cell": (C.c_int, [_P, C.c_int32, C.c_int32, C.POINTER(C.c_int32)]),

@@ -18,6 +18,10 @@ EPISODE_DTYPE = np.dtype([("episode_return", np.float32), ("length", np.int32), 
                           ("visited", np.int32), ("total_free", np.int32), ("room", np.int32),
                           ("terminated", np.int32), ("truncated", np.int32)])
 
+# columns of Engine.room_stats (nav3d_room_stat)
+ROOM_STAT_FIELDS = ("episodes", "terminated", "time_limit", "length_sum", "bumps_sum", "visited_sum", "return_centi_sum",
+                    "reserved")
+
 STATE_FIELDS = ("x", "y", "z", "facing", "visited_count", "bump_count", "step_count", "near_wall", "was_near_wall",
                 "last_bump", "done", "cells_insight_down", "last_action", "room", "episode", "return_centi")
 
@@ -138,6 +142,37 @@ class Engine:
         """float64 [n_rooms]: the exact probability of each room in a Philox reset, diff(cdf) / 2^32.  A positive weight
         below max(weights) * 2^-32 shows here as 0, as it is drawn."""
         return torch.diff(self.room_cdf(), prepend=torch.zeros(1, dtype=torch.int64, device=self.device)).double() / 2.0 ** 32
+
+    def room_stats(self, terminated: torch.Tensor, truncated: torch.Tensor, episodes: torch.Tensor,
+                   out: Optional[torch.Tensor] = None, *, check: bool = False) -> torch.Tensor:
+        """Per-room sums of the episodes that ended in one step (``terminated``, ``truncated`` uint8 [n_envs], ``episodes``
+        int32 [n_envs, 8]) or in T steps ([T, n_envs], [T, n_envs, 8]), as ``step`` and ``rollout_actions`` write them
+        (``nav3d_room_stats``).  Returns int64 [n_rooms, 8], columns ``ROOM_STAT_FIELDS``: ``out`` with the rows added
+        when given, else a fresh zeroed tensor.  Only rows whose terminated | truncated is set are read.
+
+        One kernel launch on the current stream.  ``check=False`` synchronises nothing and can be captured in a CUDA
+        graph; ``check=True`` reads the status back and raises ``Nav3dError`` if a flagged row had a room index out of
+        range or a non-finite return (such rows are never counted)."""
+        N = self.n_envs
+        T = 1 if terminated.dim() == 1 else int(terminated.shape[0])
+        lead = (N,) if terminated.dim() == 1 else (T, N)
+        self._check(terminated, torch.uint8, lead, "terminated")
+        self._check(truncated, torch.uint8, lead, "truncated")
+        self._check(episodes, torch.int32, lead + (8,), "episodes")
+        R = len(self.rooms)
+        if out is None:
+            out = torch.zeros((R, len(ROOM_STAT_FIELDS)), dtype=torch.int64, device=self.device)
+        self._check(out, torch.int64, (R, len(ROOM_STAT_FIELDS)), "out")
+        if T == 0:
+            return out
+        status = torch.empty(1, dtype=torch.uint8, device=self.device) if check else None
+        with torch.cuda.device(self.device):
+            _lib.check(self._lib.nav3d_room_stats(self._h, T, _ptr(terminated), _ptr(truncated), _ptr(episodes), _ptr(out),
+                                                  _ptr(status), self._stream()))
+        if status is not None and int(status.item()) != 0:
+            raise Nav3dError(-1, "room_stats: rows flagged done with a room index outside "
+                                 f"0..{R - 1} or a non-finite return were not counted")
+        return out
 
     def free_cell(self, room: int, k: int):
         xyz = (C.c_int32 * 3)()

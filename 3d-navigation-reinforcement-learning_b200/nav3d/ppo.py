@@ -52,7 +52,7 @@ class RecurrentPPO:
                  clip_range: float = 0.2, ent_coef: float = 0.0, vf_coef: float = 0.5, max_grad_norm: float = 0.5,
                  normalize_advantage: bool = True, seq_len: Optional[int] = None, seed: Optional[int] = 0,
                  verbose: int = 0, ops=None, device=None, policy: str = "MlpLstmPolicy", allow_tf32: bool = True,
-                 cuda_graph: bool = True, graph_chunk: int = 128, graph_update_max: int = 8192):
+                 cuda_graph: bool = True, graph_chunk: int = 128, graph_update_max: int = 8192, curriculum=None):
         if policy != "MlpLstmPolicy":
             raise ValueError("only MlpLstmPolicy is implemented (the one the reference trains)")
         self.policy_kwargs = dict(policy_kwargs or {})
@@ -64,6 +64,9 @@ class RecurrentPPO:
         self.cuda_graph, self.graph_chunk, self.graph_update_max = bool(cuda_graph), int(graph_chunk), int(graph_update_max)
         self.num_timesteps = 0
         self.n_updates = 0
+        # nav3d.curriculum.RoomCurriculum or None: observes every env step, updates the room weights after every rollout
+        self.curriculum = curriculum
+        self._curriculum_log: Dict[str, float] = {}
         self._iteration = 0
         self.seq_len = int(seq_len) if seq_len else math.gcd(self.n_steps, self.batch_size)
         if self.n_steps % self.seq_len or self.batch_size % self.seq_len:
@@ -159,6 +162,8 @@ class RecurrentPPO:
                                  step_offset=self._step_base)
         self._values[t].copy_(values)
         _, reward, dones, info = env.step(self._actions[t], out_obs=self._obs[t + 1])
+        if self.curriculum is not None:
+            self.curriculum.observe(info.terminated, info.truncated, info.episodes)
         self._rewards[t].copy_(reward)
         time_limit = (info.truncated != 0) & (info.terminated == 0)
         if sync_free or bool(time_limit.any()):
@@ -221,7 +226,13 @@ class RecurrentPPO:
             for j in range(4):
                 self._state[j].copy_(state[j])
             self._last_starts.copy_(starts)
-        n, r, l = ep.cpu().tolist()
+        if self.curriculum is not None:
+            # eager, outside any captured graph (its all-reduce); the next replay draws resets from the new table
+            self.curriculum.update()
+            n, r, l, rooms, p_min, p_max = torch.cat([ep.double(), self.curriculum.summary]).cpu().tolist()
+            self._curriculum_log = dict(curriculum_rooms=rooms, curriculum_p_min=p_min, curriculum_p_max=p_max)
+        else:
+            n, r, l = ep.cpu().tolist()
         if n > 0:
             self._ep_return_mean, self._ep_len_mean = r / n, l / n
         self._episodes_this_rollout = int(n)
@@ -412,7 +423,7 @@ class RecurrentPPO:
             rec = dict(iteration=self._iteration, total_timesteps=self.num_timesteps,
                        fps=(self.num_timesteps - steps_start) / dt, ep_rew_mean=self._ep_return_mean,
                        ep_len_mean=self._ep_len_mean, episodes=self._episodes_this_rollout, n_updates=self.n_updates,
-                       **stats)
+                       **stats, **self._curriculum_log)
             self.logger.append(rec)
             if self.verbose and self.rank == 0 and self._iteration % max(1, log_interval) == 0:
                 print("| iter {iteration:5d} | steps {total_timesteps:11d} | fps {fps:11.0f} | ep_rew_mean {ep_rew_mean:9.2f} | "
@@ -459,14 +470,18 @@ class RecurrentPPO:
 
     def save(self, path) -> Path:
         """``model.save(save_path)`` (train/Grid_Train.py:232-233): a ``.zip`` holding ``data`` (JSON hyper-parameters and
-        counters), ``policy.pth`` and ``policy.optimizer.pth`` (torch state dicts; parameter names follow sb3-contrib)."""
+        counters), ``policy.pth`` and ``policy.optimizer.pth`` (torch state dicts; parameter names follow sb3-contrib), and
+        ``curriculum.pth`` (``RoomCurriculum.state_dict``) when a curriculum is set."""
         p = _append_zip_suffix(path)
         p.parent.mkdir(parents=True, exist_ok=True)
         if self.rank != 0:
             return p
         with zipfile.ZipFile(p, "w", compression=zipfile.ZIP_STORED) as z:
             z.writestr("data", json.dumps(self._data(), indent=1))
-            for name, sd in (("policy.pth", self.policy.state_dict()), ("policy.optimizer.pth", self.optimizer.state_dict())):
+            members = [("policy.pth", self.policy.state_dict()), ("policy.optimizer.pth", self.optimizer.state_dict())]
+            if self.curriculum is not None:
+                members.append(("curriculum.pth", self.curriculum.state_dict()))
+            for name, sd in members:
                 buf = io.BytesIO()
                 torch.save(sd, buf)
                 z.writestr(name, buf.getvalue())
@@ -474,8 +489,9 @@ class RecurrentPPO:
         return p
 
     @classmethod
-    def load(cls, path, env=None, device=None, verbose: int = 0, ops=None, **overrides) -> "RecurrentPPO":
-        """``RecurrentPPO.load(model_path, env=train_env, verbose=1)`` (train/Train_Further.py:146)."""
+    def load(cls, path, env=None, device=None, verbose: int = 0, ops=None, curriculum=None, **overrides) -> "RecurrentPPO":
+        """``RecurrentPPO.load(model_path, env=train_env, verbose=1)`` (train/Train_Further.py:146).  ``curriculum``: a
+        ``RoomCurriculum`` the model uses from now on; it takes the checkpoint's curriculum state when there is one."""
         p = Path(path)
         if not p.exists():
             p = _append_zip_suffix(path)
@@ -483,12 +499,17 @@ class RecurrentPPO:
             data = json.loads(z.read("data").decode())
             policy_sd = torch.load(io.BytesIO(z.read("policy.pth")), map_location="cpu", weights_only=True)
             opt_sd = torch.load(io.BytesIO(z.read("policy.optimizer.pth")), map_location="cpu", weights_only=True)
+            cur_sd = (torch.load(io.BytesIO(z.read("curriculum.pth")), map_location="cpu", weights_only=True)
+                      if curriculum is not None and "curriculum.pth" in z.namelist() else None)
         if data.get("format_version") != FORMAT_VERSION:
             raise ValueError(f"{p}: unsupported checkpoint format {data.get('format_version')}")
         kw = {k: data[k] for k in ("learning_rate", "n_steps", "batch_size", "n_epochs", "gamma", "gae_lambda", "clip_range",
                                   "ent_coef", "vf_coef", "max_grad_norm", "normalize_advantage", "seq_len", "seed")}
         kw.update(overrides)
-        model = cls(env, policy_kwargs=data["policy_kwargs"], verbose=verbose, ops=ops, device=device, **kw)
+        model = cls(env, policy_kwargs=data["policy_kwargs"], verbose=verbose, ops=ops, device=device, curriculum=curriculum,
+                    **kw)
+        if cur_sd is not None:
+            curriculum.load_state_dict(cur_sd)
         model.policy.load_state_dict(policy_sd)
         model._flatten_grads()                                # load_state_dict keeps the parameters; re-pin the gradients
         model.optimizer.load_state_dict(opt_sd)

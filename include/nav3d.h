@@ -195,6 +195,38 @@ int nav3d_set_room_weights(nav3d_engine *e, const float *weights, uint8_t *statu
 /* DEVICE u64[n_rooms]: the current table cdf[j] as above, cdf[n_rooms-1] = 2^32.  Asynchronous device-to-device copy. */
 int nav3d_get_room_cdf(nav3d_engine *e, uint64_t *cdf, void *stream);
 
+/* ---- per-room statistics of finished episodes: what a room curriculum reads (nav3d.curriculum.RoomCurriculum).
+ * 64 bytes: one room's accumulators occupy one line.  All fields are integers, so the result does not depend on the order
+ * in which rows are added.  The sums are of the int32 fields of nav3d_episode, sign-extended, mod 2^64. */
+typedef struct {
+    uint64_t episodes;            /* rows counted */
+    uint64_t terminated;          /* of which terminated[t][i] != 0 (CubicEnv: >= 84 % explored; simpleEnv: goal reached) */
+    uint64_t time_limit;          /* of which truncated && !terminated (SB3's TimeLimit.truncated) */
+    uint64_t length_sum;          /* sum of nav3d_episode.length */
+    uint64_t bumps_sum;
+    uint64_t visited_sum;         /* mean explored fraction = visited_sum / (episodes * total_free of the room), exactly */
+    int64_t return_centi_sum;     /* sum of rint_half_even(100 * (double)episode_return); wraps mod 2^64 */
+    uint64_t reserved;            /* never written by the call (0 in a zeroed accumulator) */
+} nav3d_room_stat;
+
+/* Adds the finished episodes of T steps to acc, per room.
+ *   terminated, truncated : DEVICE u8[T][n_envs];  episodes : DEVICE nav3d_episode[T][n_envs] (4-byte aligned): what T
+ *                           nav3d_step calls or one nav3d_rollout_actions write.  All required.
+ *   acc    : DEVICE nav3d_room_stat[n_rooms], 8-byte aligned; the call ADDS to it and never zeroes it
+ *   status : DEVICE u8[1] or NULL: 1 if the call rejected a row, else 0 (not written when T == 0)
+ * Row [t][i] is counted if and only if terminated[t][i] | truncated[t][i] is nonzero, into room episodes[t][i].room; every
+ * other episode row is stale by contract and never read.  A flagged row whose room is outside 0..n_rooms-1, or whose return
+ * is not finite or has |100 * return| >= 2^63, is not counted and sets *status = 1.  The engine never writes such rows; the
+ * check exists because the buffers are the caller's.
+ * With auto_reset = 0 an env stepped on past done keeps its done flags and has its episode row rewritten every step, so the
+ * same episode is counted once per such step.
+ * Both env kinds.  Fastest when terminated and truncated have the same address mod 16 (two slices of [T][n_envs] tensors at
+ * the same index do); any alignment is accepted.  One kernel launch (plus a one-byte memset when status != NULL); no
+ * allocation, no synchronisation, no host copy: capturable in a CUDA graph.  T == 0 launches nothing; T < 0 or a NULL
+ * pointer gives NAV3D_ERR_INVALID. */
+int nav3d_room_stats(nav3d_engine *e, int32_t T, const uint8_t *terminated, const uint8_t *truncated,
+                     const nav3d_episode *episodes, nav3d_room_stat *acc, uint8_t *status, void *stream);
+
 /* The room table: replaces the per-reset text parse + free-cell scan of load_room (envs/CubicEnv.py:402-459).
  * Dense grids are uploaded once; a CUDA kernel packs each room into bit-packed occupancy words (three orientations)
  * and builds the ordered free-cell list; per-env knowledge storage is sized for the largest room.

@@ -21,6 +21,7 @@ def main():
     ap.add_argument("--epochs", type=int, default=10)
     ap.add_argument("--rooms", default="P1_training")
     ap.add_argument("--two-streams", type=int, default=1)
+    ap.add_argument("--curriculum", type=int, default=0, help="1: attach a nav3d.curriculum.RoomCurriculum to the env")
     args = ap.parse_args()
     import torch
     from nav3d import BatchedCubicEnv
@@ -30,6 +31,9 @@ def main():
                                              n_lstm_layers=1),
                      learning_rate=3e-4, n_steps=args.n_steps, batch_size=args.batch_envs * args.n_steps, n_epochs=args.epochs,
                      gamma=0.99, gae_lambda=0.95, ent_coef=0.01, vf_coef=0.5, clip_range=0.2, seed=0)
+    if args.curriculum:
+        from nav3d.curriculum import RoomCurriculum
+        m.curriculum = RoomCurriculum(env)
     m.policy.two_streams = bool(args.two_streams)
     for _ in range(2):                                   # warm-up: eager rollout, then the rollout's CUDA-graph capture
         m.collect_rollouts(); m.train()
@@ -40,7 +44,7 @@ def main():
         st = m.train(); torch.cuda.synchronize(); t2 = time.perf_counter()
         t_roll += t1 - t0; t_train += t2 - t1
     steps = args.iters * args.n_steps * args.envs
-    print(json.dumps(dict(two_streams=args.two_streams, envs=args.envs, n_steps=args.n_steps, batch_envs=args.batch_envs, epochs=args.epochs,
+    print(json.dumps(dict(two_streams=args.two_streams, curriculum=args.curriculum, envs=args.envs, n_steps=args.n_steps, batch_envs=args.batch_envs, epochs=args.epochs,
                           rollout_steps_per_s=steps / t_roll, train_steps_per_s=steps / t_train,
                           total_steps_per_s=steps / (t_roll + t_train), rollout_ms_per_step=1e3 * t_roll / (args.iters * args.n_steps),
                           minibatches=st["minibatches"], reward_mean=st["rollout_reward_mean"])))

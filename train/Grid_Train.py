@@ -24,6 +24,7 @@ import _nav3d_path  # noqa: E402,F401
 from nav3d.evaluation import EvalCallback  # noqa: E402
 from nav3d.experiment import (BASE_SEED, arch_string, checkpoint_name, dist_setup, eval_every_calls, lstm_string,  # noqa: E402
                               make_vec_env, split_segments)
+from nav3d.curriculum import RoomCurriculum  # noqa: E402
 from nav3d.ppo import RecurrentPPO  # noqa: E402
 
 random.seed(BASE_SEED)
@@ -59,6 +60,9 @@ def main(argv=None):
     ap.add_argument("--save-dir", default=SAVE_DIR)
     ap.add_argument("--eval-freq", type=int, default=0, help="steps between evaluations (default 100000; 5000000 with --native)")
     ap.add_argument("--phases", default="", help="comma-separated phase names to run (default: the PHASES list)")
+    ap.add_argument("--curriculum", action="store_true",
+                    help="draw each phase's training rooms from learning-progress weights (nav3d.curriculum.RoomCurriculum) "
+                         "instead of uniformly; evaluation is unchanged")
     args = ap.parse_args(argv)
     rank, world, local_rank = dist_setup()
     num_envs = args.num_envs or (NATIVE_NUM_ENVS if args.native else NUM_ENVS)
@@ -110,6 +114,8 @@ def main(argv=None):
                             if rank == 0:
                                 print(f"Continuing training on {phase_name}. Setting new environment.")
                             model.set_env(train_env)
+                        if args.curriculum:
+                            model.curriculum = RoomCurriculum(train_env)
                         for i, seg_steps in enumerate(segments):
                             cumulative_steps_total += seg_steps
                             if rank == 0:

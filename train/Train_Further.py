@@ -21,6 +21,7 @@ import _nav3d_path  # noqa: E402,F401
 from nav3d.evaluation import EvalCallback  # noqa: E402
 from nav3d.experiment import (BASE_SEED, continued_name, dist_setup, eval_every_calls, make_vec_env,  # noqa: E402
                               parse_view_suffix, split_segments)
+from nav3d.curriculum import RoomCurriculum  # noqa: E402
 from nav3d.ppo import RecurrentPPO  # noqa: E402
 
 random.seed(BASE_SEED)
@@ -43,6 +44,9 @@ def main(argv=None):
     ap.add_argument("--steps", type=int, default=0)
     ap.add_argument("--num-envs", type=int, default=NUM_ENVS)
     ap.add_argument("--eval-freq", type=int, default=EVAL_FREQ)
+    ap.add_argument("--curriculum", action="store_true",
+                    help="draw the training rooms from learning-progress weights (nav3d.curriculum.RoomCurriculum), starting "
+                         "afresh on this phase's rooms; evaluation is unchanged")
     args = ap.parse_args(argv)
     rank, world, local_rank = dist_setup()
     phase_name, train_path, eval_path = PHASES[0]
@@ -69,6 +73,8 @@ def main(argv=None):
         train_env = make_vec_env(train_path, ray_len, args.num_envs, 0, rank=rank, device=local_rank)
         model = RecurrentPPO.load(model_path, env=train_env, verbose=1)
         print(f"Model loaded ({model.num_timesteps} steps so far). Continuing training on {phase_name}.")
+        if args.curriculum:
+            model.curriculum = RoomCurriculum(train_env)
         for i, seg_steps in enumerate(split_segments(steps_this_phase)):
             print(f"\n--- Training {phase_name} segment {i + 1}/10 ({seg_steps} steps) ---")
             eval_callback = EvalCallback(eval_env=eval_env, best_model_save_path=best_model_dir, log_path=best_model_dir,
